@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the embedding-similarity hot path (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c1|c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c1|c2|c3|c4|c5] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: 64 queries, top-10, scored against every
 row of the HBM-resident synthetic store (SURVEY.md 8d generator).
@@ -83,6 +83,29 @@ def _tensor_peak():
         except Exception:
             pass
     return 1400.0, "fallback (B200_PROFILING.md sustained)"
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """--dump-outputs: writes each array as out_dir/<name>.npy -- integers and float64 as float64, float32 as float32 -- so
+    that two builds can be compared output for output.  Arrays share their leading dimension; when together they exceed
+    64 MB, a fixed, seeded sample of that dimension (the same rows of every array) is written, with the chosen positions
+    as sample_rows.npy."""
+    import numpy as np
+    arrays = {name: np.asarray(a) for name, a in arrays.items()}
+    arrays = {name: a.astype(np.float32 if a.dtype == np.float32 else np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = len(next(iter(arrays.values())))
+        keep = int((DUMP_LIMIT_BYTES - 4096) / (total / n + 8))     # 8 bytes a row for sample_rows, 4 KB for the headers
+        pick = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {name: a[pick] for name, a in arrays.items()}
+        arrays["sample_rows"] = pick.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -505,10 +528,11 @@ def parity_oracle_f64(store, q_host, k: int, n_queries: int, max_rows: int):
 # top-k scorer (C1 / C2 / C3, clustered variant)
 # ---------------------------------------------------------------------------------------------
 def bench_topk(ctx: Ctx, args, cfg: str, steps: int, warmup: int, variant: str = "iid", with_e2e: bool = True,
-               with_parity: bool = True, rows_override=None, store_dtype=None, cluster_rho=None):
+               with_parity: bool = True, rows_override=None, store_dtype=None, cluster_rho=None, dump_dir=None):
     """store_dtype "f64" / "f64+bf16": the same workload on a BINARY64 store -- rows kept as float64 originals (here the
     synthetic values times (1 + 1e-9 g), g ~ N(0,1): not representable in fp32 / bf16), the scan streams their rounded
-    fp32 / bf16 shadow, every exact step reads the originals; queries are float64 too."""
+    fp32 / bf16 shadow, every exact step reads the originals; queries are float64 too.
+    dump_dir: rank 0 writes the (idx, score, count) lists of the last timed step there."""
     import numpy as np
     import torch
     import vidmem_b200 as vm
@@ -599,6 +623,8 @@ def bench_topk(ctx: Ctx, args, cfg: str, steps: int, warmup: int, variant: str =
             dev_ms += ev0.elapsed_time(ev1)
         ctx.barrier()
         del flush
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"topk_idx": out[0].cpu(), "topk_score": out[1].cpu(), "topk_count": out[2].cpu()})
     stats = store.last_stats
     launches = int(stats.scan_launches) * steps
     cert = store.counters(reset=True)
@@ -744,11 +770,12 @@ def scaling_baseline(ctx: Ctx):
 # ---------------------------------------------------------------------------------------------
 # all-pairs dedup (C4)
 # ---------------------------------------------------------------------------------------------
-def bench_dedup(ctx: Ctx, args, steps: int, warmup: int, rows_override=None):
+def bench_dedup(ctx: Ctx, args, steps: int, warmup: int, rows_override=None, dump_dir=None):
     """Config C4: all-pairs dedup, 1M x 768 bf16 vs itself, threshold 0.9 (planted near-duplicates), on the run's N
     GPUs.  N > 1 goes through vm_pairs_above_sharded: tile grid dealt cyclically, ncclAllGather of counts and hit
     lists, every rank ends with the complete list (inside the timed region); the e2e leg additionally starts from
-    rows in rank 0's pinned host memory (H2D + ONE ncclBroadcast) and ends with the pairs on the host."""
+    rows in rank 0's pinned host memory (H2D + ONE ncclBroadcast) and ends with the pairs on the host.
+    dump_dir: rank 0 writes the pair list of the last timed step there."""
     import ctypes as C
     import numpy as np
     import torch
@@ -782,7 +809,6 @@ def bench_dedup(ctx: Ctx, args, steps: int, warmup: int, rows_override=None):
         h = ((oi[:m] * 1_000_003 + oj[:m]) % 2_147_483_629).sum() if m else torch.zeros((), dtype=torch.int64, device=dev)
         return m, int(h.item())
 
-    steps = max(1, min(steps, 3))
     warm = max(1, min(warmup, 1))
     for _ in range(warm):
         step()
@@ -798,6 +824,11 @@ def bench_dedup(ctx: Ctx, args, steps: int, warmup: int, rows_override=None):
     ctx.barrier()
     ms = e0.elapsed_time(e1) / steps
     hits, hsum = pair_hash()
+    if dump_dir and rank == 0:
+        m = min(hits, cap)
+        pi, pj, ps = oi[:m].cpu().numpy(), oj[:m].cpu().numpy(), os_[:m].cpu().numpy()
+        order = np.lexsort((pj, pi))                        # (i, j) order, as dedup.pairs_above returns the set
+        dump_outputs(dump_dir, {"pairs_i": pi[order], "pairs_j": pj[order], "pairs_score": ps[order]})
     # e2e: rank 0's rows come from pinned host memory every step, pairs go back to the host
     xh = None
     if rank == 0:
@@ -913,11 +944,12 @@ def bench_dedup(ctx: Ctx, args, steps: int, warmup: int, rows_override=None):
 # ---------------------------------------------------------------------------------------------
 # streaming (C5)
 # ---------------------------------------------------------------------------------------------
-def bench_streaming(ctx: Ctx, args, rounds: int, dtype=None, rows_override=None):
+def bench_streaming(ctx: Ctx, args, rounds: int, dtype=None, rows_override=None, dump_dir=None):
     """Config C5: streaming mode -- 4096-row inserts interleaved with single-query top-10 lookups over a
     10M x 384 store; p50/p99 latencies (host wall clock around synchronous host-buffer calls).
     N > 1: the store is row-sharded (10M/N rows per rank before the inserts), each 4096-row insert goes to ONE rank
-    (round-robin == least-full), every query is a collective vm_topk_sharded call (local scan, ncclAllGather, merge)."""
+    (round-robin == least-full), every query is a collective vm_topk_sharded call (local scan, ncclAllGather, merge).
+    dump_dir: rank 0 writes the lists of the last round's queries there."""
     import numpy as np
     import torch
     import vidmem_b200 as vm
@@ -927,14 +959,13 @@ def bench_streaming(ctx: Ctx, args, rounds: int, dtype=None, rows_override=None)
         rows_total = rows_override
     dt = dtype or dt
     world, rank, dev = ctx.world, ctx.rank, ctx.dev
-    rounds = max(8, min(rounds, 64))
     per_round_q = 8
     ins = 4096
     n0 = rows_total * (rank + 1) // world - rows_total * rank // world
     row_base = rank * (1 << 32)                       # global row = rank stride + local row (unique, order by rank then age)
     # growable store: exactly the resident rows are backed at the start, so the timed inserts include the store's
     # growth (new physical HBM mapped behind the resident rows; nothing is copied, addresses stay put)
-    st = EmbeddingStore(dim, n0, dt, device=ctx.local_rank, max_capacity=2 * n0 + 64 * ins)
+    st = EmbeddingStore(dim, n0, dt, device=ctx.local_rank, max_capacity=2 * n0 + max(rounds, 64) * ins)
     cap0, base0, bytes0 = st.capacity, st.rows.data_ptr(), st.resident_bytes()
     st.synth_fill(sseed, n0, row0=rows_total * rank // world)
     st.set_size(n0)
@@ -952,7 +983,7 @@ def bench_streaming(ctx: Ctx, args, rounds: int, dtype=None, rows_override=None)
     sampler = ClockSampler(ctx.local_rank, period_s=0.05)
     if rank == 0:
         sampler.start()
-    q_lat, i_lat = [], []
+    q_lat, i_lat, last_round = [], [], []
     t_all = time.perf_counter()
     for r in range(rounds):
         if r % world == rank:
@@ -961,10 +992,15 @@ def bench_streaming(ctx: Ctx, args, rounds: int, dtype=None, rows_override=None)
             i_lat.append((time.perf_counter() - t0) * 1e3)
         for qi in range(per_round_q):
             t0 = time.perf_counter()
-            st.topk(qpin[r * per_round_q + qi:r * per_round_q + qi + 1], k, comm=ctx.comm, row_offset=row_base)
+            res = st.topk(qpin[r * per_round_q + qi:r * per_round_q + qi + 1], k, comm=ctx.comm, row_offset=row_base)
             q_lat.append((time.perf_counter() - t0) * 1e3)
+            if r == rounds - 1:
+                last_round.append(res)
     wall = time.perf_counter() - t_all
     ctx.barrier()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {name: np.concatenate([res[f] for res in last_round])
+                                for f, name in enumerate(("topk_idx", "topk_score", "topk_count"))})
     clocks = sampler.stop() if rank == 0 else None
     # the planted row of the last insert must be its own best match (every rank sees the same answer)
     probe = new_rows[(rounds - 1) * ins + 17:(rounds - 1) * ins + 18].numpy()
@@ -1037,12 +1073,12 @@ def run_ours(args):
         return rec
 
     if cfg == "c4":
-        line = note("dedup", bench_dedup(ctx, args, args.steps, args.warmup, args.rows))
+        line = note("dedup", bench_dedup(ctx, args, args.steps, args.warmup, args.rows, dump_dir=args.dump_outputs))
     elif cfg == "c5":
-        line = note("streaming", bench_streaming(ctx, args, args.steps, args.c5_dtype, args.rows))
+        line = note("streaming", bench_streaming(ctx, args, args.steps, args.c5_dtype, args.rows, dump_dir=args.dump_outputs))
     else:
         line = note("topk", bench_topk(ctx, args, cfg, args.steps, args.warmup, variant=args.variant, rows_override=args.rows,
-                                       store_dtype=args.store_dtype))
+                                       store_dtype=args.store_dtype, dump_dir=args.dump_outputs))
         full = cfg in ("c2", "c3") and not args.rows and not args.only_main
         if rank == 0 and not args.no_cpu_baseline:
             cores = _use_all_host_cores()                    # torchrun pins OMP_NUM_THREADS to 1 in every worker
@@ -1063,9 +1099,10 @@ def run_ours(args):
             if world == 1 and cfg == "c2":
                 b64 = {sd: note("binary64_" + sd, bench_topk(ctx, args, cfg, min(args.steps, 20), 3, with_e2e=True, store_dtype=sd))
                        for sd in ("f64", "f64+bf16")}
-            dd = note("dedup", bench_dedup(ctx, args, args.steps, args.warmup))
-            stream = note("streaming", bench_streaming(ctx, args, args.steps))
-            stream_bf16 = note("streaming_bf16", bench_streaming(ctx, args, args.steps, "bf16"))
+            # sub-records: all-pairs steps of ~0.5 s each capped at 3, streaming rounds kept within 8..64
+            dd = note("dedup", bench_dedup(ctx, args, min(args.steps, 3), args.warmup))
+            stream = note("streaming", bench_streaming(ctx, args, max(8, min(args.steps, 64))))
+            stream_bf16 = note("streaming_bf16", bench_streaming(ctx, args, max(8, min(args.steps, 64)), "bf16"))
             if rank == 0:
                 line["clustered"] = {key: clustered[key] for key in ("value", "unit", "ms_per_step", "config", "roofline", "certification", "parity", "clocks")}
                 line["clustered"]["vs_iid"] = clustered["value"] / line["value"]
@@ -1110,7 +1147,8 @@ def torchrun_argv(gpus: int, argv, port: int):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps of the main record (c5: insert + query rounds; c4: all-pairs steps of ~0.5 s each at the default "
+                         "1M rows, so pass a small --steps with --config c4)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default=None, choices=sorted(CONFIGS) + ["c4"])
@@ -1128,7 +1166,13 @@ def main():
     ap.add_argument("--c5-dtype", default=None, choices=["f32", "bf16"])
     ap.add_argument("--store-dtype", default=None, choices=["f32", "bf16", "f64", "f64+bf16"],
                     help="store dtype override for the top-k configs (f64 / f64+bf16: binary64 store, see DESIGN.md 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the main record's timed path returned in its last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.gpus > 1 and args.impl == "ours" and "WORLD_SIZE" not in os.environ:
         # started as plain `python bench.py --gpus N`: re-launch under torchrun, one rank per GPU
         import socket

@@ -1,6 +1,6 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference functions.
 
-Run in the authoring container only (needs /root/reference):  python -m oracle.gen_golden
+Needs a checkout of the reference project (see oracle/ref_import.py):  python -m oracle.gen_golden
 The reference ships no golden vectors for this path (SURVEY.md section 4), so these
 fixtures -- outputs of the reference's own code on seeded synthetic inputs -- are what pins
 the oracle (tests/test_oracle_golden.py) and, through it, the CUDA path.

@@ -1,9 +1,10 @@
-"""Import the UNMODIFIED reference classes from /root/reference with third-party stubs.
+"""Import the UNMODIFIED reference classes from a checkout of the reference project, with third-party stubs.
 
-TEST INFRASTRUCTURE, authoring container only: /root/reference does not exist on the GPU
-box, so nothing that runs there (gpu tests, smoke(), bench.py) may import this module.  It
-is used by oracle/gen_golden.py to produce tests/golden/ fixtures and by the CPU-only test
-that re-validates the oracle against the live reference when the checkout is present.
+TEST INFRASTRUCTURE: the checkout is not part of this repository (it is looked for in
+$VIDMEM_REFERENCE_ROOT, else in oracle/_ref/), so nothing that must run from the repository
+alone (gpu tests, smoke(), bench.py) may import this module.  It is used by
+oracle/gen_golden.py to produce tests/golden/ fixtures and by the CPU-only tests that
+compare with the live reference when a checkout is present.
 
 Missing third-party modules (langchain*, neo4j, sentence_transformers: SURVEY.md 8c) are
 replaced with empty stand-ins in sys.modules; the reference's own code is executed as-is.
@@ -16,7 +17,7 @@ import sys
 import tempfile
 import types
 
-REFERENCE_ROOT = os.environ.get("VIDMEM_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("VIDMEM_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def available() -> bool:

@@ -5,7 +5,7 @@ import os
 import numpy as np
 import pytest
 
-from oracle import oracle, synth
+from oracle import oracle, ref_import, synth
 
 
 def _load(golden_dir, name):
@@ -147,9 +147,8 @@ def test_synth_numpy_equals_c():
     assert np.array_equal(v, np.round(v)) and np.abs(v).max() <= 127
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference checkout not present")
+@pytest.mark.skipif(not ref_import.available(), reason="reference checkout not present (see oracle/ref_import.py)")
 def test_oracle_against_live_reference():
-    from oracle import ref_import
     X = synth.synth_rows(77, 0, 120, 96)
     Q = synth.synth_queries(78, 3, 96, 77, 120)
     store = {f"c{i}": [float(v) for v in X[i]] for i in range(len(X))}
