@@ -70,7 +70,7 @@ enum {
     VM_FLAG_ASYNC = 1,       /* do not synchronise (device outputs only) */
     VM_FLAG_FORCE_EXACT = 2, /* skip the fast scan: binary64 scan of every row (slow, always exact) */
     VM_FLAG_FORCE_SIMT = 4,  /* use the CUDA-core scan kernel even where the tcgen05 kernel applies */
-    VM_FLAG_FORCE_TC = 8,    /* use the tcgen05/TMA scan kernel even for small query batches */
+    VM_FLAG_FORCE_TC = 8,    /* accepted and ignored: the tcgen05/TMA scan kernel is the default wherever it applies */
     VM_FLAG_TIMING = 16,     /* bracket the scan kernel with CUDA events on `stream` (see vm_store_last_scan_ms);
                                 also launches the call's kernels without programmatic overlap */
     VM_FLAG_NO_SPLIT = 32,   /* bf16 store: feed the query as ONE bf16 term (scan error bound 2^-8) */

@@ -69,6 +69,33 @@ static constexpr int MAX_DEVICES = 64;
 static constexpr int COLLECT_CAP = 4096;         // rows per query the collect pass may gather
 static constexpr int FLAG_INTERNAL_CAPTURE = 1 << 30;  // set by the CUDA-graph path while capturing
 
+// The top-k results of a batch as one contiguous block [idx nq*k i64 | score nq*k f64 | count nq i32], so that one
+// copy moves all three arrays: the host readback, the all-gather and the peer-exchange slot all use this layout.
+struct ResultBlock {
+    int64_t *idx;
+    double *score;
+    int32_t *count;
+    static ResultBlock at(void *base, int nq, int k)
+    {
+        char *b = (char *)base;
+        return {(int64_t *)b, (double *)(b + (size_t)nq * k * 8), (int32_t *)(b + (size_t)nq * k * 16)};
+    }
+    // the rows of query q0 onwards in three separate [nq][k], [nq][k], [nq] arrays
+    ResultBlock from(int q0, int k) const { return {idx + (size_t)q0 * k, score + (size_t)q0 * k, count + q0}; }
+};
+static constexpr size_t result_bytes(int nq, int k) { return (size_t)nq * k * 16 + (size_t)nq * 4; }
+// one rank's block of the cross-shard exchange: the result block padded to 8 bytes
+static constexpr size_t packed_bytes(int nq, int k) { return (result_bytes(nq, k) + 7) & ~(size_t)7; }
+
+// copies a result block from (pinned) host memory into the caller's three arrays
+static void unpack_to_host(const void *pack, int nq, int k, const ResultBlock &out)
+{
+    const ResultBlock p = ResultBlock::at(const_cast<void *>(pack), nq, k);
+    memcpy(out.idx, p.idx, (size_t)nq * k * 8);
+    memcpy(out.score, p.score, (size_t)nq * k * 8);
+    memcpy(out.count, p.count, (size_t)nq * 4);
+}
+
 struct DeviceGuard {
     int prev = -1;
     bool ok = true;
@@ -101,7 +128,7 @@ struct Workspace {
     int lists_max = 0;
     Buf q_raw, q_f32, q_bf16, seed, cand, merged, o_idx, flags, col_thr, col_cnt, col_buf, xs, xr, xc, taken, gather_send, gather_recv, misc, ubuf, done, scnt, sel_inc;
     int32_t *h_uncert = nullptr;  // pinned
-    unsigned char *h_pack = nullptr;  // pinned: packed [idx | score | count] of one batch
+    unsigned char *h_pack = nullptr;  // pinned: the ResultBlock of one batch
     unsigned char *h_q = nullptr;     // pinned: host queries of one batch
     void release()
     {
@@ -167,7 +194,7 @@ struct vm_store {
 };
 
 // exchange buffer of one rank: two result slots + a generation flag
-static constexpr size_t XCHG_SLOT_BYTES = ((size_t)MAXQ * MAXK * 16 + (size_t)MAXQ * 4 + 255) & ~(size_t)255;
+static constexpr size_t XCHG_SLOT_BYTES = (result_bytes(MAXQ, MAXK) + 255) & ~(size_t)255;
 static constexpr size_t XCHG_FLAG_OFF = 2 * XCHG_SLOT_BYTES;
 static constexpr size_t XCHG_BYTES = XCHG_FLAG_OFF + 256;
 
@@ -247,8 +274,7 @@ static int ws_prepare(vm_store *s)
     ENS(w.q_bf16, (size_t)2 * MAXQ * s->ld * 2);  // hi terms, then lo terms (split query)
     ENS(w.cand, (size_t)lists * MAXQ * (MAXK > SCAN_SLAB ? MAXK : SCAN_SLAB) * 8);  // per-CTA lists / dumped tiles / slabs
     ENS(w.merged, (size_t)MAXQ * MAXK * 8);
-    // one contiguous block [idx | score | count] so a host caller gets its results with ONE copy
-    ENS(w.o_idx, (size_t)MAXQ * MAXK * 16 + (size_t)MAXQ * 4 + 64);
+    ENS(w.o_idx, result_bytes(MAXQ, MAXK) + 64);
     ENS(w.flags, (size_t)(MAXQ + 2) * 4);
     // per-CTA maxima [256][64] + published per-query bounds [64] + their counter [64] + union-buffer counters [64] (scan_tc.cu);
     // zeroed as one block by the normalise kernel
@@ -267,7 +293,7 @@ static int ws_prepare(vm_store *s)
     ENS(w.taken, (size_t)MAXQ * XCTAS * MAXK);
 #undef ENS
     VM_CUDA_CHECK(cudaMallocHost((void **)&w.h_uncert, 64));
-    VM_CUDA_CHECK(cudaMallocHost((void **)&w.h_pack, (size_t)MAXQ * MAXK * 16 + (size_t)MAXQ * 4 + 64));
+    VM_CUDA_CHECK(cudaMallocHost((void **)&w.h_pack, result_bytes(MAXQ, MAXK) + 64));
     VM_CUDA_CHECK(cudaMallocHost((void **)&w.h_q, (size_t)MAXQ * s->dim * 8));
     w.ready = true;
     return VM_OK;
@@ -332,7 +358,7 @@ static int store_new(vm_store **out, int device, int dim, int dtype, int64_t cap
         if (cudaMalloc((void **)&s->extreme, 4) != cudaSuccess || cudaMemset(s->extreme, 0, 4) != cudaSuccess ||
             cudaMalloc((void **)&s->cum, 64) != cudaSuccess || cudaMemset(s->cum, 0, 64) != cudaSuccess) {
             set_error("store allocation failed");
-            delete s;
+            vm_store_destroy(s);
             return VM_ERR_OOM;
         }
     }
@@ -346,18 +372,16 @@ extern "C" int vm_store_create(vm_store **out, int device, int dim, int dtype, i
     if (rc != VM_OK) return rc;
     vm_store *s = *out;
     DeviceGuard g(device);
+    s->owns = true;
     size_t bytes = (size_t)capacity * s->ld * dtype_size(dtype);
     cudaError_t e = cudaMalloc(&s->rows, bytes);
     if (e == cudaSuccess) e = cudaMalloc((void **)&s->inv_norms, (size_t)capacity * 4);
     if (e != cudaSuccess) {
         set_error("store allocation of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
-        if (s->rows) cudaFree(s->rows);
-        if (s->extreme) cudaFree(s->extreme);
-        delete s;
+        vm_store_destroy(s);
         *out = nullptr;
         return VM_ERR_OOM;
     }
-    s->owns = true;
     return VM_OK;
 }
 
@@ -658,8 +682,6 @@ extern "C" int vm_store_clear(vm_store *s)
 }
 
 // ---- top-k ------------------------------------------------------------------------------------
-// One rank's block of the cross-shard exchange: [idx nq*k i64 | score nq*k f64 | count nq i32, padded to 8 bytes]
-static inline size_t packed_bytes(int nq, int k) { return (size_t)nq * k * 16 + (((size_t)nq * 4 + 7) & ~(size_t)7); }
 extern "C" size_t vm_topk_packed_bytes(int nq, int k) { return nq > 0 && k > 0 ? packed_bytes(nq, k) : 0; }
 
 namespace {
@@ -670,22 +692,15 @@ struct TopkCall {
     double min_score;
     int score_mode, sum_mode, flags;
     int64_t row_offset;
-    // device destinations for this batch
-    int64_t *d_idx;
-    double *d_score;
-    int32_t *d_count;
+    ResultBlock d;  // device destinations for this batch
     cudaStream_t st;
     vm_topk_stats *stats;
     // optional host destinations: results are copied there inside the same synchronisation that reads
     // the uncertified-query counter (one stream sync per batch on the host-buffer path)
-    int64_t *h_idx = nullptr;
-    double *h_score = nullptr;
-    int32_t *h_count = nullptr;
+    ResultBlock h = {};
 };
 }  // namespace
 
-// Host-output path: the batch's device results are one contiguous block [idx | score | count]
-// (see ws_prepare); one D2H copy into pinned memory, then plain host copies into the caller's arrays.
 // Result wait of the synchronous (host-buffer) calls.  cudaStreamSynchronize may park the thread for work longer
 // than ~1 ms and then pays a 0.1-0.2 ms wake-up; a top-k call is latency-critical and short, so poll instead
 // (VIDMEM_SYNC=block restores the blocking wait, e.g. on oversubscribed hosts).
@@ -713,22 +728,29 @@ static cudaError_t wait_stream(cudaStream_t st, const vm_store *s = nullptr)
     }
 }
 
+// Host-output path: the batch's device results are one ResultBlock (see ws_prepare); one D2H copy into pinned
+// memory, then plain host copies into the caller's arrays.
 static int pack_out_enqueue(const TopkCall &c)
 {
-    const size_t bytes = (size_t)c.nq * c.k * 16 + (size_t)c.nq * 4;
-    VM_CUDA_CHECK(cudaMemcpyAsync(c.s->ws.h_pack, c.d_idx, bytes, cudaMemcpyDeviceToHost, c.st));
+    VM_CUDA_CHECK(cudaMemcpyAsync(c.s->ws.h_pack, c.d.idx, result_bytes(c.nq, c.k), cudaMemcpyDeviceToHost, c.st));
     return VM_OK;
 }
-static void pack_out_finish(const TopkCall &c)
+
+// candidate-list length of the tcgen05 scan for top-k (0: k is too large for it)
+static int tc_list_len(int k) { return k <= 16 ? 32 : (k <= 48 ? 64 : 0); }
+
+// queries per scan pass: 64, or fewer when 64 normalised queries of this dimension do not fit the
+// tcgen05 kernel's shared memory (e.g. 16 for a 1536-d fp32 store)
+static int queries_per_pass(const vm_store *s, int k, int flags)
 {
-    const size_t seg = (size_t)c.nq * c.k * 8;
-    const unsigned char *p = c.s->ws.h_pack;
-    memcpy(c.h_idx, p, seg);
-    memcpy(c.h_score, p + seg, seg);
-    memcpy(c.h_count, p + 2 * seg, (size_t)c.nq * 4);
+    const int kp = tc_list_len(k);
+    if (!(flags & (VM_FLAG_FORCE_EXACT | VM_FLAG_FORCE_SIMT)) && kp)
+        for (int nq = 64; nq >= 16; nq -= 16)
+            if (scan_tc_supported(s->dtype, s->dim, nq, kp)) return nq;
+    return MAXQ;
 }
 
-// One batch of <= MAXQ queries; results land in c.d_* (device).  May synchronise the stream
+// One batch of <= MAXQ queries; results land in c.d (device).  May synchronise the stream
 // (unless VM_FLAG_ASYNC) to learn whether any query needs the exact re-scan.
 static int topk_batch(const TopkCall &c)
 {
@@ -743,7 +765,7 @@ static int topk_batch(const TopkCall &c)
         VM_CUDA_CHECK(cudaMemcpyAsync(w.q_raw.p, w.h_q, qbytes, cudaMemcpyHostToDevice, st));
         q_dev = w.q_raw.p;
     }
-    FinalizeArgs fin{c.k, c.min_score, c.score_mode, c.row_offset, c.d_idx, c.d_score, c.d_count};
+    FinalizeArgs fin{c.k, c.min_score, c.score_mode, c.row_offset, c.d.idx, c.d.score, c.d.count};
     ExactArgs ex{s->exact_rows(), s->inv_norms, s->exact_dtype(), s->ld, s->dim, s->size, q_dev, c.q_dtype, c.nq, c.k, c.sum_mode,
                  nullptr, (double *)w.xs.p, (uint32_t *)w.xr.p, (int32_t *)w.xc.p, (uint8_t *)w.taken.p, XCTAS, fin, s->cum,
                  (int *)w.done.p};
@@ -754,7 +776,7 @@ static int topk_batch(const TopkCall &c)
     // choose the scan kernel
     int kernel = 0, kp = 0;
     if (!(c.flags & VM_FLAG_FORCE_EXACT) && s->size > 0) {
-        int kp_tc = c.k <= 16 ? 32 : (c.k <= 48 ? 64 : 0);
+        int kp_tc = tc_list_len(c.k);
         int kp_simt = c.k <= 24 ? (c.k + 8 > 16 ? ((c.k + 8 + 7) & ~7) : 16) : 0;
         bool tc_ok = kp_tc > 0 && scan_tc_supported(s->dtype, s->dim, c.nq, kp_tc);
         // The tcgen05 scan is the default at every size: it streams big shards at the HBM roofline (the CUDA-core
@@ -770,10 +792,10 @@ static int topk_batch(const TopkCall &c)
         int rc = k_exact(ex, st, false);
         if (rc != VM_OK) return rc;
         launches += 2;
-        if (c.h_idx) {
+        if (c.h.idx) {
             if ((rc = pack_out_enqueue(c)) != VM_OK) return rc;
             VM_CUDA_CHECK(wait_stream(st, s));
-            pack_out_finish(c);
+            unpack_to_host(w.h_pack, c.nq, c.k, c.h);
         }
         if (c.stats) { c.stats->scan_kernel = 0; c.stats->scan_launches += launches; }
         return VM_OK;
@@ -887,7 +909,7 @@ static int topk_batch(const TopkCall &c)
         n_uncert = -1;
     } else {
         VM_CUDA_CHECK(cudaMemcpyAsync(w.h_uncert, uncert, 4, cudaMemcpyDeviceToHost, st));
-        if (c.h_idx && (rc = pack_out_enqueue(c)) != VM_OK) return rc;
+        if (c.h.idx && (rc = pack_out_enqueue(c)) != VM_OK) return rc;
         VM_CUDA_CHECK(wait_stream(st, s));
         n_uncert = *w.h_uncert;
         n_full = 0;
@@ -906,12 +928,12 @@ static int topk_batch(const TopkCall &c)
                 if (rc != VM_OK) return rc;
                 launches += 1;
             }
-            if (c.h_idx) {
+            if (c.h.idx) {
                 if ((rc = pack_out_enqueue(c)) != VM_OK) return rc;
                 VM_CUDA_CHECK(wait_stream(st, s));
             }
         }
-        if (c.h_idx) pack_out_finish(c);
+        if (c.h.idx) unpack_to_host(w.h_pack, c.nq, c.k, c.h);
     }
     if (c.stats) {
         c.stats->scan_kernel = kernel;
@@ -924,6 +946,117 @@ static int topk_batch(const TopkCall &c)
         c.stats->scan_variant = kernel == 2 ? sinfo.variant : 0;
     }
     return VM_OK;
+}
+
+// topk_graph: the call is not one for the graph path
+static constexpr int GRAPH_SKIPPED = 1;
+
+// Captures the pipeline of the one-batch host-buffer call c into cache entry ge: H2D of the pinned queries ->
+// normalise -> scan -> select/rescore -> D2H of the uncertified-query count and of the result block.
+static int graph_capture(const TopkCall &c, vm_store::GraphEntry *ge)
+{
+    vm_store *s = c.s;
+    Workspace &w = s->ws;
+    vm_topk_stats cs{};
+    TopkCall cc = c;
+    cc.queries = w.q_raw.p; cc.q_mem = VM_MEM_DEVICE; cc.flags |= VM_FLAG_ASYNC | FLAG_INTERNAL_CAPTURE;
+    cc.d = ResultBlock::at(w.o_idx.p, c.nq, c.k); cc.st = s->gstream; cc.stats = &cs;
+    const size_t qbytes = (size_t)c.nq * s->dim * dtype_size(c.q_dtype);
+    cudaGraph_t graph = nullptr;
+    VM_CUDA_CHECK(cudaStreamBeginCapture(s->gstream, cudaStreamCaptureModeRelaxed));
+    int rc = VM_OK;
+    if (cudaMemcpyAsync(w.q_raw.p, w.h_q, qbytes, cudaMemcpyHostToDevice, s->gstream) != cudaSuccess) rc = VM_ERR_CUDA;
+    if (rc == VM_OK) rc = topk_batch(cc);
+    if (rc == VM_OK && cudaMemcpyAsync(w.h_pack, cc.d.idx, result_bytes(c.nq, c.k), cudaMemcpyDeviceToHost, s->gstream) != cudaSuccess)
+        rc = VM_ERR_CUDA;
+    cudaError_t ce = cudaStreamEndCapture(s->gstream, &graph);
+    if (rc != VM_OK || ce != cudaSuccess || !graph) {
+        if (graph) cudaGraphDestroy(graph);
+        if (rc == VM_OK) { set_error("graph capture failed: %s", cudaGetErrorString(ce)); rc = VM_ERR_CUDA; }
+        cudaGetLastError();
+        return rc;
+    }
+    ce = cudaGraphInstantiate(&ge->exec, graph, 0);
+    cudaGraphDestroy(graph);
+    if (ce != cudaSuccess) { ge->exec = nullptr; set_error("cudaGraphInstantiate failed: %s", cudaGetErrorString(ce)); return VM_ERR_CUDA; }
+    ge->version = s->version; ge->nq = c.nq; ge->k = c.k; ge->flags = c.flags; ge->score_mode = c.score_mode;
+    ge->sum_mode = c.sum_mode; ge->q_dtype = c.q_dtype; ge->min_score = c.min_score; ge->row_offset = c.row_offset; ge->stats = cs;
+    return VM_OK;
+}
+
+// CUDA-graph fast path: one graph launch runs the whole pipeline of the call (graph_capture), and the
+// device-conditional exact re-scan is replaced by a host re-run of the rare uncertified batch.  Host buffers, one
+// batch, caller on the legacy default stream (the graph runs on a library-owned blocking stream, which the legacy
+// stream orders with).  The graph bakes in row count and TMA descriptors, so it is keyed on the store version.
+// c describes the whole call; returns GRAPH_SKIPPED when the call must take the batch loop instead.
+static int topk_graph(const TopkCall &c, int out_mem, bool sharded, const ResultBlock &out)
+{
+    vm_store *s = c.s;
+    Workspace &w = s->ws;
+    static const bool no_graph = getenv("VIDMEM_NO_GRAPH") != nullptr;
+    // capturing costs a few hundred microseconds: only worth it for a store that is being queried, not
+    // one that is mutated every few calls (streaming inserts)
+    if (s->seen_version == s->version) { if (s->stable_calls < 1 << 20) ++s->stable_calls; }
+    else { s->seen_version = s->version; s->stable_calls = 0; }
+    if (no_graph || s->stable_calls < 16 || sharded || c.st != nullptr || c.q_mem != VM_MEM_HOST || out_mem != VM_MEM_HOST ||
+        (c.flags & (VM_FLAG_ASYNC | VM_FLAG_TIMING | VM_FLAG_FORCE_EXACT)) || s->size == 0 ||
+        c.nq > queries_per_pass(s, c.k, c.flags))
+        return GRAPH_SKIPPED;
+    if (!s->gstream) VM_CUDA_CHECK(cudaStreamCreate(&s->gstream));
+    vm_store::GraphEntry *ge = nullptr;
+    for (auto &e : s->graphs)
+        if (e.exec && e.version == s->version && e.nq == c.nq && e.k == c.k && e.flags == c.flags && e.score_mode == c.score_mode &&
+            e.sum_mode == c.sum_mode && e.q_dtype == c.q_dtype && e.row_offset == c.row_offset &&
+            memcmp(&e.min_score, &c.min_score, sizeof(double)) == 0) { ge = &e; break; }  // bitwise: a NaN bound must match itself
+    if (!ge) {  // capture into the oldest entry
+        ge = &s->graphs[s->graph_next];
+        s->graph_next = (s->graph_next + 1) & 3;
+        if (ge->exec) { cudaGraphExecDestroy(ge->exec); ge->exec = nullptr; }
+        const int rc = graph_capture(c, ge);
+        if (rc != VM_OK) return rc;
+    }
+    memcpy(w.h_q, c.queries, (size_t)c.nq * s->dim * dtype_size(c.q_dtype));
+    ++s->n_batches; s->n_queries += c.nq;
+    VM_CUDA_CHECK(cudaGraphLaunch(ge->exec, s->gstream));
+    VM_CUDA_CHECK(wait_stream(s->gstream, s));
+    const int uncertified = ge->stats.scan_kernel != 0 ? *w.h_uncert : 0;  // the exact-only pipeline writes no count
+    if (uncertified > 0) {
+        // some query was not certified: run this batch through the plain path (collect pass / exact scan)
+        TopkCall rerun = c;
+        rerun.d = ResultBlock::at(w.o_idx.p, c.nq, c.k); rerun.st = s->gstream; rerun.h = out;
+        return topk_batch(rerun);
+    }
+    unpack_to_host(w.h_pack, c.nq, c.k, out);
+    if (c.stats) { *c.stats = ge->stats; c.stats->uncertified = uncertified; }
+    return VM_OK;
+}
+
+// offset of this rank's result slot of exchange generation gen in the peer-mapped buffer (two slots alternate)
+static size_t xchg_slot_off(unsigned long long gen) { return (size_t)(gen & 1) * XCHG_SLOT_BYTES; }
+
+// where the local pass of a batch writes its results: this rank's exchange slot (p2p), the all-gather send buffer
+// (NCCL), the caller's arrays (device outputs) or the workspace block (host outputs)
+static ResultBlock batch_dest(vm_store *s, const vm_comm *comm, bool sharded, int out_mem, const ResultBlock &out, int nb, int k)
+{
+    if (sharded && comm->p2p) return ResultBlock::at((char *)comm->peer[comm->rank] + xchg_slot_off(comm->gen), nb, k);
+    if (sharded) return ResultBlock::at(s->ws.gather_send.p, nb, k);
+    return out_mem == VM_MEM_DEVICE ? out : ResultBlock::at(s->ws.o_idx.p, nb, k);
+}
+
+// Exchanges the local results of one sharded batch between the ranks -- peer-mapped slots, or ONE all-gather of the
+// result blocks -- and merges them into m
+static int exchange_merge(vm_store *s, vm_comm *comm, int nb, int k, const ResultBlock &m, cudaStream_t st)
+{
+    if (comm->p2p) {
+        const int rc = k_p2p_publish((char *)comm->peer[comm->rank] + XCHG_FLAG_OFF, comm->gen, st);
+        if (rc != VM_OK) return rc;
+        return k_merge_topk_p2p(comm->peer, comm->nranks, xchg_slot_off(comm->gen), XCHG_FLAG_OFF, comm->gen, nb, k, m.idx, m.score,
+                                m.count, st);
+    }
+    const Workspace &w = s->ws;
+    VM_NCCL_CHECK(g_nccl.AllGather(w.gather_send.p, w.gather_recv.p, packed_bytes(nb, k), /*ncclInt8*/ 0, comm->nccl, st));
+    const ResultBlock r = ResultBlock::at(w.gather_recv.p, nb, k);
+    return k_merge_topk_lists(r.idx, r.score, r.count, packed_bytes(nb, k), comm->nranks, nb, k, m.idx, m.score, m.count, st);
 }
 
 static int topk_common(vm_store *s, vm_comm *comm, int64_t row_offset, const void *queries, int q_dtype, int q_mem, int nq,
@@ -945,181 +1078,43 @@ static int topk_common(vm_store *s, vm_comm *comm, int64_t row_offset, const voi
     VM_REQUIRE(g.ok, VM_ERR_CUDA, "cannot select device %d", s->device);
     int rc = ws_prepare(s);
     if (rc != VM_OK) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    Workspace &w = s->ws;
-    const size_t qrow = (size_t)s->dim * dtype_size(q_dtype);
     const bool sharded = comm && comm->nranks > 1;
+    const ResultBlock out{out_idx, out_score, out_count};
+    const TopkCall call{s, queries, q_dtype, q_mem, nq, k, min_score, score_mode, sum_mode, flags, row_offset, {}, (cudaStream_t)stream,
+                        stats};
+    if ((rc = topk_graph(call, out_mem, sharded, out)) != GRAPH_SKIPPED) return rc;
 
-    // ---- CUDA-graph fast path: one graph launch for H2D -> normalise -> scan -> select/rescore ->
-    // (device-conditional exact re-scan) -> packed D2H.  Host buffers, one batch, caller on the legacy
-    // default stream (the graph runs on a library-owned blocking stream, which the legacy stream orders
-    // with).  The graph bakes in row count and TMA descriptors, so it is keyed on the store version.
-    static const bool no_graph = getenv("VIDMEM_NO_GRAPH") != nullptr;
-    // capturing costs a few hundred microseconds: only worth it for a store that is being queried, not
-    // one that is mutated every few calls (streaming inserts)
-    if (s->seen_version == s->version) { if (s->stable_calls < 1 << 20) ++s->stable_calls; }
-    else { s->seen_version = s->version; s->stable_calls = 0; }
-    if (!no_graph && s->stable_calls >= 16 && !sharded && st == nullptr && q_mem == VM_MEM_HOST && out_mem == VM_MEM_HOST && nq <= MAXQ &&
-        !(flags & (VM_FLAG_ASYNC | VM_FLAG_TIMING | VM_FLAG_FORCE_EXACT)) && s->size > 0) {
-        if (!s->gstream) VM_CUDA_CHECK(cudaStreamCreate(&s->gstream));
-        vm_store::GraphEntry *ge = nullptr;
-        for (auto &e : s->graphs)
-            if (e.exec && e.version == s->version && e.nq == nq && e.k == k && e.flags == flags && e.score_mode == score_mode &&
-                e.sum_mode == sum_mode && e.q_dtype == q_dtype && e.row_offset == row_offset &&
-                memcmp(&e.min_score, &min_score, sizeof(double)) == 0) { ge = &e; break; }  // bitwise: a NaN bound must match itself
-        int bq_g = MAXQ;
-        if (!(flags & VM_FLAG_FORCE_SIMT)) {
-            const int kp_tc = k <= 16 ? 32 : (k <= 48 ? 64 : 0);
-            bq_g = 0;
-            if (kp_tc)
-                for (int cand = 64; cand >= 16; cand -= 16)
-                    if (scan_tc_supported(s->dtype, s->dim, cand, kp_tc)) { bq_g = cand; break; }
-            if (bq_g == 0) bq_g = MAXQ;
-        }
-        if (nq <= bq_g) {
-            const size_t qbytes = (size_t)nq * qrow, obytes = (size_t)nq * k * 16 + (size_t)nq * 4;
-            int64_t *ws_idx = (int64_t *)w.o_idx.p;
-            double *ws_score = (double *)((char *)w.o_idx.p + (size_t)nq * k * 8);
-            int32_t *ws_count = (int32_t *)((char *)w.o_idx.p + (size_t)nq * k * 16);
-            if (!ge) {
-                ge = &s->graphs[s->graph_next];
-                s->graph_next = (s->graph_next + 1) & 3;
-                if (ge->exec) { cudaGraphExecDestroy(ge->exec); ge->exec = nullptr; }
-                vm_topk_stats cs{};
-                cudaGraph_t graph = nullptr;
-                VM_CUDA_CHECK(cudaStreamBeginCapture(s->gstream, cudaStreamCaptureModeRelaxed));
-                rc = VM_OK;
-                if (cudaMemcpyAsync(w.q_raw.p, w.h_q, qbytes, cudaMemcpyHostToDevice, s->gstream) != cudaSuccess) rc = VM_ERR_CUDA;
-                if (rc == VM_OK) {
-                    TopkCall c{s, w.q_raw.p, q_dtype, VM_MEM_DEVICE, nq, k, min_score, score_mode, sum_mode,
-                               flags | VM_FLAG_ASYNC | FLAG_INTERNAL_CAPTURE,
-                               row_offset, ws_idx, ws_score, ws_count, s->gstream, &cs};
-                    rc = topk_batch(c);
-                }
-                if (rc == VM_OK && cudaMemcpyAsync(w.h_pack, ws_idx, obytes, cudaMemcpyDeviceToHost, s->gstream) != cudaSuccess) rc = VM_ERR_CUDA;
-
-                cudaError_t ce = cudaStreamEndCapture(s->gstream, &graph);
-                if (rc != VM_OK || ce != cudaSuccess || !graph) {
-                    if (graph) cudaGraphDestroy(graph);
-                    if (rc == VM_OK) { set_error("graph capture failed: %s", cudaGetErrorString(ce)); rc = VM_ERR_CUDA; }
-                    cudaGetLastError();
-                    return rc;
-                }
-                ce = cudaGraphInstantiate(&ge->exec, graph, 0);
-                cudaGraphDestroy(graph);
-                if (ce != cudaSuccess) { ge->exec = nullptr; set_error("cudaGraphInstantiate failed: %s", cudaGetErrorString(ce)); return VM_ERR_CUDA; }
-                ge->version = s->version; ge->nq = nq; ge->k = k; ge->flags = flags; ge->score_mode = score_mode;
-                ge->sum_mode = sum_mode; ge->q_dtype = q_dtype; ge->min_score = min_score; ge->row_offset = row_offset; ge->stats = cs;
-            }
-            memcpy(w.h_q, queries, qbytes);
-            ++s->n_batches; s->n_queries += nq;
-            VM_CUDA_CHECK(cudaGraphLaunch(ge->exec, s->gstream));
-            VM_CUDA_CHECK(wait_stream(s->gstream, s));
-            if (ge->stats.scan_kernel != 0 && *w.h_uncert > 0) {
-                // some query was not certified: run this batch through the plain path (collect pass / exact scan)
-                TopkCall c{s, queries, q_dtype, VM_MEM_HOST, nq, k, min_score, score_mode, sum_mode, flags, row_offset,
-                           ws_idx, ws_score, ws_count, s->gstream, stats};
-                c.h_idx = out_idx; c.h_score = out_score; c.h_count = out_count;
-                return topk_batch(c);
-            }
-            const size_t seg = (size_t)nq * k * 8;
-            memcpy(out_idx, w.h_pack, seg);
-            memcpy(out_score, w.h_pack + seg, seg);
-            memcpy(out_count, w.h_pack + 2 * seg, (size_t)nq * 4);
-            if (stats) {
-                *stats = ge->stats;
-                stats->uncertified = ge->stats.scan_kernel != 0 ? *w.h_uncert : 0;
-            }
-            return VM_OK;
-        }
-    }
-
-    // queries per scan pass: 64, or fewer when 64 normalised queries of this dimension do not fit the
-    // tcgen05 kernel's shared memory (e.g. 16 for a 1536-d fp32 store)
-    int bq = MAXQ;
-    if (!(flags & (VM_FLAG_FORCE_EXACT | VM_FLAG_FORCE_SIMT))) {
-        const int kp_tc = k <= 16 ? 32 : (k <= 48 ? 64 : 0);
-        if (kp_tc)
-            for (int cand = 64; cand >= 16; cand -= 16)
-                if (scan_tc_supported(s->dtype, s->dim, cand, kp_tc)) { bq = cand; break; }
-    }
+    Workspace &w = s->ws;
+    const int bq = queries_per_pass(s, k, flags);
     for (int q0 = 0; q0 < nq; q0 += bq) {
-        int nb = nq - q0 < bq ? nq - q0 : bq;
-        // where this batch's local results go
-        bool direct = out_mem == VM_MEM_DEVICE && !sharded;
-        // workspace block of this batch: [idx nb*k | score nb*k | count nb], contiguous
-        int64_t *ws_idx = (int64_t *)w.o_idx.p;
-        double *ws_score = (double *)((char *)w.o_idx.p + (size_t)nb * k * 8);
-        int32_t *ws_count = (int32_t *)((char *)w.o_idx.p + (size_t)nb * k * 16);
-        int64_t *d_idx = direct ? out_idx + (size_t)q0 * k : ws_idx;
-        double *d_score = direct ? out_score + (size_t)q0 * k : ws_score;
-        int32_t *d_count = direct ? out_count + q0 : ws_count;
-        const bool p2p = sharded && comm->p2p;
-        unsigned long long gen = 0;
-        size_t slot_off = 0;
-        if (p2p) {
-            // peer-memory exchange: results go straight into this rank's slot of the symmetric buffer
-            gen = ++comm->gen;
-            slot_off = (size_t)(gen & 1) * XCHG_SLOT_BYTES;
-            char *slot = (char *)comm->peer[comm->rank] + slot_off;
-            d_idx = (int64_t *)slot;
-            d_score = (double *)(slot + (size_t)nb * k * 8);
-            d_count = (int32_t *)(slot + (size_t)nb * k * 16);
+        const int nb = nq - q0 < bq ? nq - q0 : bq;
+        const ResultBlock out_b = out.from(q0, k);
+        if (sharded && comm->p2p) {
+            ++comm->gen;  // a fresh exchange slot and flag value for this batch
         } else if (sharded) {
-            // pack [idx | score | count] contiguously so ONE all-gather moves the batch
-            size_t seg = (size_t)nb * k * 8;
-            size_t per_rank = packed_bytes(nb, k);
-            rc = w.gather_send.ensure(per_rank);
-            if (rc == VM_OK) rc = w.gather_recv.ensure(per_rank * comm->nranks);
-            if (rc != VM_OK) return rc;
-            d_idx = (int64_t *)w.gather_send.p;
-            d_score = (double *)((char *)w.gather_send.p + seg);
-            d_count = (int32_t *)((char *)w.gather_send.p + 2 * seg);
+            if ((rc = w.gather_send.ensure(packed_bytes(nb, k))) != VM_OK) return rc;
+            if ((rc = w.gather_recv.ensure(packed_bytes(nb, k) * comm->nranks)) != VM_OK) return rc;
         }
-        // Sharded call with host outputs: enqueue the local pass without a host round trip (uncertified queries
-        // are settled by the device-conditional binary64 scan), so scan -> exchange -> merge -> one packed D2H run
-        // back to back and the ranks reach the all-gather together; the only synchronisation is the final one.
-        const bool sharded_host = sharded && out_mem == VM_MEM_HOST && !(flags & VM_FLAG_ASYNC);
-        TopkCall c{s, (const char *)queries + (size_t)q0 * qrow, q_dtype, q_mem, nb, k, min_score, score_mode, sum_mode,
-                   sharded_host ? (flags | VM_FLAG_ASYNC) : flags, row_offset, d_idx, d_score,
-                   d_count, st, stats};
-        const bool host_direct = out_mem == VM_MEM_HOST && !sharded && !(flags & VM_FLAG_ASYNC);
-        if (host_direct) { c.h_idx = out_idx + (size_t)q0 * k; c.h_score = out_score + (size_t)q0 * k; c.h_count = out_count + q0; }
-        rc = topk_batch(c);
-        if (rc != VM_OK) return rc;
-        if (sharded) {
-            bool dd = out_mem == VM_MEM_DEVICE;
-            int64_t *m_idx = dd ? out_idx + (size_t)q0 * k : ws_idx;
-            double *m_score = dd ? out_score + (size_t)q0 * k : ws_score;
-            int32_t *m_count = dd ? out_count + q0 : ws_count;
-            if (p2p) {
-                rc = k_p2p_publish((char *)comm->peer[comm->rank] + XCHG_FLAG_OFF, gen, st);
-                if (rc == VM_OK)
-                    rc = k_merge_topk_p2p(comm->peer, comm->nranks, slot_off, XCHG_FLAG_OFF, gen, nb, k, m_idx, m_score, m_count, st);
-            } else {
-                size_t seg = (size_t)nb * k * 8;
-                size_t per_rank = packed_bytes(nb, k);
-                VM_NCCL_CHECK(g_nccl.AllGather(w.gather_send.p, w.gather_recv.p, per_rank, /*ncclInt8*/ 0, comm->nccl, st));
-                const char *rb = (const char *)w.gather_recv.p;
-                rc = k_merge_topk_lists(rb, rb + seg, rb + 2 * seg, per_rank, comm->nranks, nb, k, m_idx, m_score, m_count, st);
-            }
-            if (rc != VM_OK) return rc;
-            if (stats) stats->scan_launches += 2;
-            d_idx = m_idx; d_score = m_score; d_count = m_count;
+        TopkCall c = call;
+        c.queries = (const char *)queries + (size_t)q0 * s->dim * dtype_size(q_dtype);
+        c.nq = nb;
+        c.d = batch_dest(s, comm, sharded, out_mem, out_b, nb, k);
+        if (out_mem == VM_MEM_HOST) {
+            // Sharded call with host outputs: enqueue the local pass without a host round trip (uncertified queries
+            // are settled by the device-conditional binary64 scan), so scan -> exchange -> merge -> one packed D2H run
+            // back to back and the ranks reach the exchange together; the only synchronisation is the final one.
+            if (sharded) c.flags |= VM_FLAG_ASYNC;
+            else c.h = out_b;
         }
-        if (sharded_host) {
-            // merged results sit in the contiguous workspace block [idx | score | count]: one D2H into pinned memory
-            const size_t seg = (size_t)nb * k * 8;
-            VM_CUDA_CHECK(cudaMemcpyAsync(w.h_pack, ws_idx, 2 * seg + (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
-            VM_CUDA_CHECK(wait_stream(st, s));
-            memcpy(out_idx + (size_t)q0 * k, w.h_pack, seg);
-            memcpy(out_score + (size_t)q0 * k, w.h_pack + seg, seg);
-            memcpy(out_count + q0, w.h_pack + 2 * seg, (size_t)nb * 4);
-        } else if (out_mem == VM_MEM_HOST && !host_direct) {
-            VM_CUDA_CHECK(cudaMemcpyAsync(out_idx + (size_t)q0 * k, d_idx, (size_t)nb * k * 8, cudaMemcpyDeviceToHost, st));
-            VM_CUDA_CHECK(cudaMemcpyAsync(out_score + (size_t)q0 * k, d_score, (size_t)nb * k * 8, cudaMemcpyDeviceToHost, st));
-            VM_CUDA_CHECK(cudaMemcpyAsync(out_count + q0, d_count, (size_t)nb * 4, cudaMemcpyDeviceToHost, st));
-            VM_CUDA_CHECK(wait_stream(st, s));
+        if ((rc = topk_batch(c)) != VM_OK) return rc;
+        if (!sharded) continue;
+        const ResultBlock ws = ResultBlock::at(w.o_idx.p, nb, k);
+        if ((rc = exchange_merge(s, comm, nb, k, out_mem == VM_MEM_DEVICE ? out_b : ws, c.st)) != VM_OK) return rc;
+        if (stats) stats->scan_launches += 2;
+        if (out_mem == VM_MEM_HOST) {
+            VM_CUDA_CHECK(cudaMemcpyAsync(w.h_pack, ws.idx, result_bytes(nb, k), cudaMemcpyDeviceToHost, c.st));
+            VM_CUDA_CHECK(wait_stream(c.st, s));
+            unpack_to_host(w.h_pack, nb, k, out_b);
         }
     }
     return VM_OK;
@@ -1149,10 +1144,8 @@ extern "C" int vm_merge_topk_lists(int device, const int64_t *idx_dev, const dou
     VM_REQUIRE(idx_dev && score_dev && count_dev && out_idx_dev && out_score_dev && out_count_dev, VM_ERR_BADARG, "NULL buffer");
     VM_REQUIRE(nlists >= 1 && nq >= 1 && k >= 1, VM_ERR_BADARG, "bad shape");
     DeviceGuard g(device);
-    // three separate arrays: each has its own per-list stride, so run with stride == idx stride
-    // only when they coincide (nq*k*8 for idx/score, nq*4 for count) -> use a packed copy-free
-    // trick: launch with per-array strides equalised by passing count through a widened view.
-    // Simplest correct path: the kernel takes ONE stride, so gather the counts to that stride.
+    // the merge kernel steps from list to list with one stride for all three arrays, so the counts ([nlists][nq]) are
+    // copied out to the stride of the idx and score lists
     size_t stride = (size_t)nq * k * 8;
     VM_REQUIRE(device >= 0 && device < MAX_DEVICES, VM_ERR_BADARG, "device index %d outside [0, %d)", device, MAX_DEVICES);
     static thread_local Buf cnt_wide_dev[MAX_DEVICES];  // scratch is device memory: one per device
@@ -1171,9 +1164,8 @@ extern "C" int vm_merge_topk_packed(int device, const void *packed_dev, int nlis
     VM_REQUIRE(packed_dev && out_idx_dev && out_score_dev && out_count_dev, VM_ERR_BADARG, "NULL buffer");
     VM_REQUIRE(nlists >= 1 && nq >= 1 && k >= 1, VM_ERR_BADARG, "bad shape");
     DeviceGuard g(device);
-    const char *rb = (const char *)packed_dev;
-    const size_t seg = (size_t)nq * k * 8;
-    return k_merge_topk_lists(rb, rb + seg, rb + 2 * seg, packed_bytes(nq, k), nlists, nq, k, out_idx_dev, out_score_dev,
+    const ResultBlock r = ResultBlock::at(const_cast<void *>(packed_dev), nq, k);
+    return k_merge_topk_lists(r.idx, r.score, r.count, packed_bytes(nq, k), nlists, nq, k, out_idx_dev, out_score_dev,
                               out_count_dev, (cudaStream_t)stream);
 }
 

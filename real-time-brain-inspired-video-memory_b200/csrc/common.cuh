@@ -52,6 +52,20 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
+// Raises Kernel's dynamic shared-memory limit to `bytes` on the current device.  The attribute is per device; it is
+// set on a device's first launch only, so later launches pay no driver call.
+template <auto Kernel>
+static inline cudaError_t max_smem_once(int bytes)
+{
+    static bool set[64] = {};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess || set[dev & 63]) return e;
+    e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess) set[dev & 63] = true;
+    return e;
+}
+
 // ---- candidate keys --------------------------------------------------------------------
 // A candidate is one u64: high word = order-preserving image of the fp32 score, low word =
 // ~row.  Larger key == better candidate (higher score, then LOWER row), keys are unique per

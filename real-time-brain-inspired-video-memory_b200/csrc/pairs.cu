@@ -545,7 +545,6 @@ int k_pairs_above(int device, const void *x, int dtype, int64_t n, int dim, int 
     if (rc != VM_OK) return rc;
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    const int dev_idx = device & 63;
 #ifdef VIDMEM_TRIAGE_KERNELS
     static const bool one_cta = getenv("VIDMEM_PAIRS_1CTA") != nullptr;  // perf triage builds only: force the 1-CTA kernel
 #else
@@ -561,12 +560,10 @@ int k_pairs_above(int device, const void *x, int dtype, int64_t n, int dim, int 
         if (my_tiles < pairs) pairs = my_tiles;
         const int grid = (int)(2 * pairs);
         if (dtype == VM_F32) {
-            static bool set[64] = {};  // the attribute is per device
-            if (!set[dev_idx]) { VM_CUDA_CHECK(cudaFuncSetAttribute(pairs_tc2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); set[dev_idx] = true; }
+            VM_CUDA_CHECK((max_smem_once<pairs_tc2_kernel<true>>(227 * 1024)));
             pairs_tc2_kernel<true><<<grid, P_THREADS, smem, st>>>(tmA, p);
         } else {
-            static bool set[64] = {};  // the attribute is per device
-            if (!set[dev_idx]) { VM_CUDA_CHECK(cudaFuncSetAttribute(pairs_tc2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); set[dev_idx] = true; }
+            VM_CUDA_CHECK((max_smem_once<pairs_tc2_kernel<false>>(227 * 1024)));
             pairs_tc2_kernel<false><<<grid, P_THREADS, smem, st>>>(tmA, p);
         }
     } else {
@@ -576,12 +573,10 @@ int k_pairs_above(int device, const void *x, int dtype, int64_t n, int dim, int 
         const long long my_tiles = (p.total_tiles + nparts - 1) / nparts;
         const int grid = (int)(my_tiles < sms ? my_tiles : sms);
         if (dtype == VM_F32) {
-            static bool set[64] = {};  // the attribute is per device
-            if (!set[dev_idx]) { VM_CUDA_CHECK(cudaFuncSetAttribute(pairs_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); set[dev_idx] = true; }
+            VM_CUDA_CHECK((max_smem_once<pairs_tc_kernel<true>>(227 * 1024)));
             pairs_tc_kernel<true><<<grid, P_THREADS, smem, st>>>(tmA, tmB, p);
         } else {
-            static bool set[64] = {};  // the attribute is per device
-            if (!set[dev_idx]) { VM_CUDA_CHECK(cudaFuncSetAttribute(pairs_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); set[dev_idx] = true; }
+            VM_CUDA_CHECK((max_smem_once<pairs_tc_kernel<false>>(227 * 1024)));
             pairs_tc_kernel<false><<<grid, P_THREADS, smem, st>>>(tmA, tmB, p);
         }
     }

@@ -205,10 +205,9 @@ static int launch_one(const ScanArgs &a, int q0)
 {
     size_t smem = (size_t)QB * a.ld * 4 + (size_t)SIMT_WARPS * QB * 32 * 8;
     VM_REQUIRE(smem <= 160 * 1024, VM_ERR_UNSUPPORTED, "SIMT scan: dim %d too large for %d queries per pass", a.dim, QB);
-    auto kern = scan_simt_kernel<T, QB>;
-    if (smem > 48 * 1024) VM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<a.ctas, SIMT_WARPS * 32, smem, a.stream>>>((const T *)a.rows, a.inv_norms, a.n, a.ld, a.queries, q0, a.nq,
-                                                       a.kp, a.cand);
+    VM_CUDA_CHECK((max_smem_once<scan_simt_kernel<T, QB>>(160 * 1024)));
+    scan_simt_kernel<T, QB><<<a.ctas, SIMT_WARPS * 32, smem, a.stream>>>((const T *)a.rows, a.inv_norms, a.n, a.ld, a.queries, q0,
+                                                                         a.nq, a.kp, a.cand);
     VM_CUDA_CHECK(cudaGetLastError());
     return VM_OK;
 }

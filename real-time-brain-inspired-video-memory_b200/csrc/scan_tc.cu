@@ -573,9 +573,6 @@ int launch_scan_tc(const ScanArgs &a, const void *queries_store_dtype, uint32_t 
                              (uint32_t)L.nq_pad);
     if (rc != VM_OK) return rc;
     const int num_tiles = (int)((a.n + TC_BLOCK_M - 1) / TC_BLOCK_M);
-    int dev_idx = 0;
-    VM_CUDA_CHECK(cudaGetDevice(&dev_idx));
-    dev_idx &= 63;
     const bool dump = a.dump && !sc;
     if (sc || dump || a.ctas > 256) { seed_tab = nullptr; seed_ctr = nullptr; }
     CollectArgs col{};
@@ -605,11 +602,7 @@ int launch_scan_tc(const ScanArgs &a, const void *queries_store_dtype, uint32_t 
 #endif
 #define LAUNCH_TC(TF, DU, SP)                                                                                                \
     do {                                                                                                                   \
-        static bool set[64] = {}; /* the attribute is per device */                                                        \
-        if (!set[dev_idx]) {                                                                                               \
-            VM_CUDA_CHECK(cudaFuncSetAttribute(scan_tc_kernel<TF, DU, SP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); \
-            set[dev_idx] = true;                                                                                           \
-        }                                                                                                                  \
+        VM_CUDA_CHECK((max_smem_once<scan_tc_kernel<TF, DU, SP>>(227 * 1024)));                                              \
         LAUNCH_IMPL(TF, DU, SP);                                                                                           \
     } while (0)
     if (a.dtype == VM_F32) { if (dump) LAUNCH_TC(true, true, false); else LAUNCH_TC(true, false, false); }

@@ -3,6 +3,8 @@
 // uncertified queries, the cross-shard merge and the cross-query max-by-id merge.
 #include "common.cuh"
 
+#include <type_traits>
+
 namespace vm {
 
 // =========================================================================================
@@ -1439,11 +1441,7 @@ __global__ void cosine_pairs_kernel(const void *__restrict__ a, const void *__re
 int k_merge_candidates(const uint64_t *cand, int lists, int nq, int kp, uint64_t *merged, cudaStream_t st)
 {
     size_t smem = (size_t)lists * kp * sizeof(uint64_t) + (size_t)lists * sizeof(uint32_t) + 16;
-    static bool attr_set_dev[64] = {};  /* the attribute is per device */ int dev_idx_ = 0; cudaGetDevice(&dev_idx_); bool &attr_set = attr_set_dev[dev_idx_ & 63];
-    if (!attr_set) {
-        VM_CUDA_CHECK(cudaFuncSetAttribute(merge_candidates_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        attr_set = true;
-    }
+    VM_CUDA_CHECK((max_smem_once<merge_candidates_kernel>(200 * 1024)));
     VM_REQUIRE(smem <= 200 * 1024, VM_ERR_UNSUPPORTED, "candidate merge: %d lists x %d exceeds shared memory", lists, kp);
     merge_candidates_kernel<<<nq, MERGE_THREADS, smem, st>>>(cand, lists, nq, kp, merged);
     VM_CUDA_CHECK(cudaGetLastError());
@@ -1451,32 +1449,42 @@ int k_merge_candidates(const uint64_t *cand, int lists, int nq, int kp, uint64_t
 }
 
 
+// Calls f(neu) with neu a std::integral_constant<bool, Neumaier summation>, so f instantiates the matching
+// <NEUMAIER> kernel.
+template <typename F>
+static int with_sum_mode(int sum_mode, F &&f)
+{
+    return sum_mode == VM_SUM_NEUMAIER ? f(std::true_type{}) : f(std::false_type{});
+}
+
+// Calls f(neu, (T *)nullptr) for the summation mode (as above) and the row type T of a row dtype.
+template <typename F>
+static int with_row_type(int dtype, int sum_mode, F &&f)
+{
+    auto by_sum = [&](auto *tag) { return with_sum_mode(sum_mode, [&](auto neu) { return f(neu, tag); }); };
+    if (dtype == VM_F32) return by_sum((float *)nullptr);
+    if (dtype == VM_F64) return by_sum((double *)nullptr);
+    return by_sum((__nv_bfloat16 *)nullptr);
+}
+
 int k_rescore(const RescoreArgs &a, cudaStream_t st, const int *incomplete)
 {
-#define LAUNCH_RS(NEU, T)                                                                                              \
-    do {                                                                                                               \
-        static bool attr_set_dev[64] = {};  /* the attribute is per device */ int dev_idx_ = 0; cudaGetDevice(&dev_idx_); bool &attr_set = attr_set_dev[dev_idx_ & 63];                                                                                  \
-        if (!attr_set) {                                                                                               \
-            VM_CUDA_CHECK(cudaFuncSetAttribute(rescore_kernel<NEU, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024)); \
-            attr_set = true;                                                                                           \
-        }                                                                                                              \
-        rescore_kernel<NEU, T><<<a.nq, RS_THREADS, smem, st>>>(a.merged, a.kp, (const T *)a.rows, a.inv_norms, a.ld, a.dim, \
-                                                               a.n_rows, a.queries, a.q_dtype, a.eps, a.fin, a.flags,    \
-                                                               a.uncertified_count, chunk, a.extreme, a.collect_thr, a.cum, incomplete);         \
-    } while (0)
     // column chunk: whole rows when kp rows fit in RS_SMEM_ROW_BYTES, else a multiple of 8 columns
     const int ssz = a.dtype == VM_F64 ? 8 : 4;  // staged element size (StageOf)
     int chunk = RS_SMEM_ROW_BYTES / (ssz * a.kp) - 1;
     chunk &= ~7;
     if (chunk > a.ld) chunk = a.ld;
     const size_t smem = (size_t)chunk * sizeof(double) + (size_t)a.kp * (chunk + 1) * ssz + 16;
-    bool neu = a.sum_mode == VM_SUM_NEUMAIER;
-    if (a.dtype == VM_F32) { if (neu) LAUNCH_RS(true, float); else LAUNCH_RS(false, float); }
-    else if (a.dtype == VM_F64) { if (neu) LAUNCH_RS(true, double); else LAUNCH_RS(false, double); }
-    else { if (neu) LAUNCH_RS(true, __nv_bfloat16); else LAUNCH_RS(false, __nv_bfloat16); }
-#undef LAUNCH_RS
-    VM_CUDA_CHECK(cudaGetLastError());
-    return VM_OK;
+    return with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
+        using T = std::remove_pointer_t<decltype(tag)>;
+        constexpr bool NEU = decltype(neu)::value;
+        VM_CUDA_CHECK((max_smem_once<rescore_kernel<NEU, T>>(160 * 1024)));
+        rescore_kernel<NEU, T><<<a.nq, RS_THREADS, smem, st>>>(a.merged, a.kp, (const T *)a.rows, a.inv_norms, a.ld, a.dim,
+                                                               a.n_rows, a.queries, a.q_dtype, a.eps, a.fin, a.flags,
+                                                               a.uncertified_count, chunk, a.extreme, a.collect_thr, a.cum, incomplete);
+        VM_CUDA_CHECK(cudaGetLastError());
+        return VM_OK;
+    });
 }
 
 
@@ -1523,26 +1531,16 @@ int k_select_rescore(const SelectArgs &sa, const RescoreArgs &a, cudaStream_t st
     if (!select_rescore_fits(src.lists, src.list_len, a.kp, a.dtype, a.dim, a.ld)) return VM_ERR_UNSUPPORTED;
     src.band_cap = select_band_cap(src.key_cap, src.lists, a.kp, a.dtype, a.dim, a.ld);
     const size_t smem = select_rescore_base_smem(src.key_cap, src.lists, a.kp, a.dtype, a.dim, a.ld) + (size_t)src.band_cap * 12;
-#define LAUNCH_SR(NEU, T)                                                                                              \
-    do {                                                                                                               \
-        static bool attr_set_dev[64] = {};                                                                             \
-        int dev_idx_ = 0;                                                                                              \
-        cudaGetDevice(&dev_idx_);                                                                                      \
-        if (!attr_set_dev[dev_idx_ & 63]) {                                                                            \
-            VM_CUDA_CHECK(cudaFuncSetAttribute(select_rescore_kernel<NEU, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 180 * 1024)); \
-            attr_set_dev[dev_idx_ & 63] = true;                                                                        \
-        }                                                                                                              \
-        VM_CUDA_CHECK(launch_pdl(select_rescore_kernel<NEU, T>, dim3(a.nq), dim3(SR_THREADS), smem, st, pdl, src, a.nq, a.kp, \
-                                 (const T *)a.rows, a.ld, a.dim, a.n_rows, a.queries, a.q_dtype, a.eps, a.fin, a.flags,      \
-                                 a.uncertified_count, a.extreme, a.collect_thr, a.cum, a.inv_norms));                       \
-    } while (0)
-    const bool neu = a.sum_mode == VM_SUM_NEUMAIER;
-    if (a.dtype == VM_F32) { if (neu) LAUNCH_SR(true, float); else LAUNCH_SR(false, float); }
-    else if (a.dtype == VM_F64) { if (neu) LAUNCH_SR(true, double); else LAUNCH_SR(false, double); }
-    else { if (neu) LAUNCH_SR(true, __nv_bfloat16); else LAUNCH_SR(false, __nv_bfloat16); }
-#undef LAUNCH_SR
-    VM_CUDA_CHECK(cudaGetLastError());
-    return VM_OK;
+    return with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
+        using T = std::remove_pointer_t<decltype(tag)>;
+        constexpr bool NEU = decltype(neu)::value;
+        VM_CUDA_CHECK((max_smem_once<select_rescore_kernel<NEU, T>>(180 * 1024)));
+        VM_CUDA_CHECK(launch_pdl(select_rescore_kernel<NEU, T>, dim3(a.nq), dim3(SR_THREADS), smem, st, pdl, src, a.nq, a.kp,
+                                 (const T *)a.rows, a.ld, a.dim, a.n_rows, a.queries, a.q_dtype, a.eps, a.fin, a.flags,
+                                 a.uncertified_count, a.extreme, a.collect_thr, a.cum, a.inv_norms));
+        VM_CUDA_CHECK(cudaGetLastError());
+        return VM_OK;
+    });
 }
 
 // slab-mode selection alone (rows too large for the fused kernel): merged [nq][kp], incomplete [nq]
@@ -1563,25 +1561,15 @@ int k_collect_rescore(const uint64_t *buf, const int *cnt, int cap, const Rescor
     const int stage_rows = staged <= 200 * 1024 ? 32 : 0;
     const size_t smem = stage_rows ? staged : head + (size_t)cap * (8 + 8 + 4) + 32;
     VM_REQUIRE(smem <= 200 * 1024, VM_ERR_UNSUPPORTED, "collect pass: buffer of %d rows exceeds shared memory", cap);
-#define LAUNCH_CR(NEU, T)                                                                                               \
-    do {                                                                                                                \
-        static bool attr_set_dev[64] = {};                                                                              \
-        int dev_idx_ = 0;                                                                                               \
-        cudaGetDevice(&dev_idx_);                                                                                       \
-        if (!attr_set_dev[dev_idx_ & 63]) {                                                                             \
-            VM_CUDA_CHECK(cudaFuncSetAttribute(collect_rescore_kernel<NEU, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024)); \
-            attr_set_dev[dev_idx_ & 63] = true;                                                                         \
-        }                                                                                                               \
-        collect_rescore_kernel<NEU, T><<<a.nq, CR_THREADS, smem, st>>>(buf, cnt, cap, (const T *)a.rows, a.ld, a.dim, a.queries, \
-                                                                       a.q_dtype, a.fin, a.flags, a.uncertified_count, a.nq, a.cum, stage_rows); \
-    } while (0)
-    const bool neu = a.sum_mode == VM_SUM_NEUMAIER;
-    if (a.dtype == VM_F32) { if (neu) LAUNCH_CR(true, float); else LAUNCH_CR(false, float); }
-    else if (a.dtype == VM_F64) { if (neu) LAUNCH_CR(true, double); else LAUNCH_CR(false, double); }
-    else { if (neu) LAUNCH_CR(true, __nv_bfloat16); else LAUNCH_CR(false, __nv_bfloat16); }
-#undef LAUNCH_CR
-    VM_CUDA_CHECK(cudaGetLastError());
-    return VM_OK;
+    return with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
+        using T = std::remove_pointer_t<decltype(tag)>;
+        constexpr bool NEU = decltype(neu)::value;
+        VM_CUDA_CHECK((max_smem_once<collect_rescore_kernel<NEU, T>>(200 * 1024)));
+        collect_rescore_kernel<NEU, T><<<a.nq, CR_THREADS, smem, st>>>(buf, cnt, cap, (const T *)a.rows, a.ld, a.dim, a.queries,
+                                                                       a.q_dtype, a.fin, a.flags, a.uncertified_count, a.nq, a.cum, stage_rows);
+        VM_CUDA_CHECK(cudaGetLastError());
+        return VM_OK;
+    });
 }
 
 // a.flags == NULL: every query (VM_FLAG_FORCE_EXACT), scan + merge kernel.  a.flags != NULL: the conditional fix-up
@@ -1592,29 +1580,19 @@ int k_exact(const ExactArgs &a, cudaStream_t st, bool pdl)
     VM_REQUIRE((size_t)a.dim * sizeof(double) <= 40 * 1024, VM_ERR_UNSUPPORTED, "exact scan: dim %d too large", a.dim);
     const size_t smem = (size_t)((a.dim + 1) & ~1) * sizeof(double) + (size_t)3 * 128 * XS_PITCH + 16;  // query + three staged chunks
     const bool conditional = a.flags != nullptr && a.done_ctr != nullptr;
-#define LAUNCH_EX(NEU, T)                                                                                               \
-    do {                                                                                                                \
-        static bool attr_set_dev[64] = {};                                                                              \
-        int dev_idx_ = 0;                                                                                               \
-        cudaGetDevice(&dev_idx_);                                                                                       \
-        if (!attr_set_dev[dev_idx_ & 63]) {                                                                             \
-            VM_CUDA_CHECK(cudaFuncSetAttribute(exact_scan_kernel<NEU, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024)); \
-            attr_set_dev[dev_idx_ & 63] = true;                                                                         \
-        }                                                                                                               \
-        VM_CUDA_CHECK(launch_pdl(exact_scan_kernel<NEU, T>, dim3(a.ctas), dim3(XS_THREADS), smem, st, pdl && conditional, (const T *)a.rows, \
-                                 a.inv_norms, a.n, a.ld, a.dim, a.queries, a.q_dtype, a.nq, a.flags, a.k, a.xlist_score, a.xlist_row, \
-                                 a.xlist_cnt, a.cum, conditional ? a.done_ctr : (int *)nullptr, a.fin, a.taken));       \
-    } while (0)
-    bool neu = a.sum_mode == VM_SUM_NEUMAIER;
-    if (a.dtype == VM_F32) { if (neu) LAUNCH_EX(true, float); else LAUNCH_EX(false, float); }
-    else if (a.dtype == VM_F64) { if (neu) LAUNCH_EX(true, double); else LAUNCH_EX(false, double); }
-    else { if (neu) LAUNCH_EX(true, __nv_bfloat16); else LAUNCH_EX(false, __nv_bfloat16); }
-#undef LAUNCH_EX
-    VM_CUDA_CHECK(cudaGetLastError());
-    if (!conditional) {
-        exact_merge_kernel<<<a.nq, 256, 0, st>>>(a.xlist_score, a.xlist_row, a.xlist_cnt, a.ctas, a.nq, a.k, a.flags, a.fin, a.taken);
+    const int rc = with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
+        using T = std::remove_pointer_t<decltype(tag)>;
+        constexpr bool NEU = decltype(neu)::value;
+        VM_CUDA_CHECK((max_smem_once<exact_scan_kernel<NEU, T>>(200 * 1024)));
+        VM_CUDA_CHECK(launch_pdl(exact_scan_kernel<NEU, T>, dim3(a.ctas), dim3(XS_THREADS), smem, st, pdl && conditional, (const T *)a.rows,
+                                 a.inv_norms, a.n, a.ld, a.dim, a.queries, a.q_dtype, a.nq, a.flags, a.k, a.xlist_score, a.xlist_row,
+                                 a.xlist_cnt, a.cum, conditional ? a.done_ctr : (int *)nullptr, a.fin, a.taken));
         VM_CUDA_CHECK(cudaGetLastError());
-    }
+        return VM_OK;
+    });
+    if (rc != VM_OK || conditional) return rc;
+    exact_merge_kernel<<<a.nq, 256, 0, st>>>(a.xlist_score, a.xlist_row, a.xlist_cnt, a.ctas, a.nq, a.k, a.flags, a.fin, a.taken);
+    VM_CUDA_CHECK(cudaGetLastError());
     return VM_OK;
 }
 
@@ -1624,11 +1602,7 @@ int k_merge_topk_lists(const void *idx, const void *score, const void *count, si
     int total = lists * k;
     VM_REQUIRE(total <= 4096, VM_ERR_UNSUPPORTED, "merge_topk_lists: lists*k = %d > 4096", total);
     size_t smem = (size_t)total * (8 + 8 + 4);
-    static bool attr_set_dev[64] = {};  /* the attribute is per device */ int dev_idx_ = 0; cudaGetDevice(&dev_idx_); bool &attr_set = attr_set_dev[dev_idx_ & 63];
-    if (!attr_set) {
-        VM_CUDA_CHECK(cudaFuncSetAttribute(merge_topk_lists_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-        attr_set = true;
-    }
+    VM_CUDA_CHECK((max_smem_once<merge_topk_lists_kernel>(100 * 1024)));
     merge_topk_lists_kernel<<<nq, 256, smem, st>>>((const char *)idx, (const char *)score, (const char *)count, stride_bytes, lists, nq, k,
                                                   out_idx, out_score, out_count);
     VM_CUDA_CHECK(cudaGetLastError());
@@ -1651,13 +1625,7 @@ int k_merge_topk_p2p(void *const *peers, int nranks, size_t slot_off, size_t fla
     PeerPtrs pp{};
     for (int r = 0; r < nranks; ++r) pp.p[r] = (const unsigned char *)peers[r];
     const size_t smem = (size_t)total * (8 + 8 + 4);
-    static bool attr_set_dev[64] = {};
-    int dev_idx_ = 0;
-    cudaGetDevice(&dev_idx_);
-    if (!attr_set_dev[dev_idx_ & 63]) {
-        VM_CUDA_CHECK(cudaFuncSetAttribute(merge_topk_p2p_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-        attr_set_dev[dev_idx_ & 63] = true;
-    }
+    VM_CUDA_CHECK((max_smem_once<merge_topk_p2p_kernel>(100 * 1024)));
     merge_topk_p2p_kernel<<<nq, 256, smem, st>>>(pp, nranks, slot_off, flag_off, gen, nq, k, out_idx, out_score, out_count);
     VM_CUDA_CHECK(cudaGetLastError());
     return VM_OK;
@@ -1669,11 +1637,7 @@ int k_merge_max_by_id(const int64_t *idx, const double *score, const int32_t *co
     int total = nq * k;
     VM_REQUIRE(total <= 4096, VM_ERR_UNSUPPORTED, "merge_max_by_id: nq*k = %d > 4096", total);
     size_t smem = (size_t)total * (8 + 8 + 4);
-    static bool attr_set_dev[64] = {};  /* the attribute is per device */ int dev_idx_ = 0; cudaGetDevice(&dev_idx_); bool &attr_set = attr_set_dev[dev_idx_ & 63];
-    if (!attr_set) {
-        VM_CUDA_CHECK(cudaFuncSetAttribute(merge_max_by_id_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-        attr_set = true;
-    }
+    VM_CUDA_CHECK((max_smem_once<merge_max_by_id_kernel>(100 * 1024)));
     merge_max_by_id_kernel<<<1, 256, smem, st>>>(idx, score, count, nq, k, k2, out_idx, out_score, out_count);
     VM_CUDA_CHECK(cudaGetLastError());
     return VM_OK;
@@ -1684,10 +1648,11 @@ int k_cosine_pairs(const void *a, const void *b, int dtype, int64_t n, int dim, 
 {
     if (n <= 0) return VM_OK;
     int grid = (int)((n + 127) / 128);
-    if (sum_mode == VM_SUM_NEUMAIER) cosine_pairs_kernel<true><<<grid, 128, 0, st>>>(a, b, dtype, n, dim, zero_rule, out);
-    else cosine_pairs_kernel<false><<<grid, 128, 0, st>>>(a, b, dtype, n, dim, zero_rule, out);
-    VM_CUDA_CHECK(cudaGetLastError());
-    return VM_OK;
+    return with_sum_mode(sum_mode, [&](auto neu) -> int {
+        cosine_pairs_kernel<decltype(neu)::value><<<grid, 128, 0, st>>>(a, b, dtype, n, dim, zero_rule, out);
+        VM_CUDA_CHECK(cudaGetLastError());
+        return VM_OK;
+    });
 }
 
 }  // namespace vm
