@@ -31,10 +31,7 @@ int k_normalize_queries(const void *q, int q_dtype, int nq, int nq_pad, int dim,
                         int32_t *zero_me, uint32_t *zero_tab, int zero_tab_n, int tf32_round, int split, bool pdl, cudaStream_t st);
 int k_synth_fill(void *rows, int dtype, uint64_t seed, int64_t row0, int64_t n, int dim, int ld, uint64_t dup_period,
                  cudaStream_t st);
-int k_merge_candidates(const uint64_t *cand, int lists, int nq, int kp, uint64_t *merged, cudaStream_t st);
 
-int k_slab_top(const SelectArgs &sa, int nq, int kp, uint64_t *merged, int *incomplete, cudaStream_t st);
-int k_rescore(const RescoreArgs &a, cudaStream_t st, const int *incomplete);
 int k_select_rescore(const SelectArgs &sa, const RescoreArgs &a, cudaStream_t st, bool pdl);
 bool select_rescore_fits(int lists, int list_len, int kp, int dtype, int dim, int ld);
 int k_collect_rescore(const uint64_t *buf, const int *cnt, int cap, const RescoreArgs &a, cudaStream_t st);
@@ -126,14 +123,14 @@ struct Buf {
 struct Workspace {
     bool ready = false;
     int lists_max = 0;
-    Buf q_raw, q_f32, q_bf16, seed, cand, merged, o_idx, flags, col_thr, col_cnt, col_buf, xs, xr, xc, taken, gather_send, gather_recv, misc, ubuf, done, scnt, sel_inc;
+    Buf q_raw, q_f32, q_bf16, seed, cand, o_idx, flags, col_thr, col_cnt, col_buf, xs, xr, xc, taken, gather_send, gather_recv, misc, ubuf, done, scnt;
     int32_t *h_uncert = nullptr;  // pinned
     unsigned char *h_pack = nullptr;  // pinned: the ResultBlock of one batch
     unsigned char *h_q = nullptr;     // pinned: host queries of one batch
     void release()
     {
-        Buf *all[] = {&q_raw, &q_f32, &q_bf16, &seed, &cand, &merged, &o_idx, &flags, &col_thr, &col_cnt, &col_buf, &xs, &xr, &xc, &taken,
-                      &gather_send, &gather_recv, &misc, &ubuf, &done, &scnt, &sel_inc};
+        Buf *all[] = {&q_raw, &q_f32, &q_bf16, &seed, &cand, &o_idx, &flags, &col_thr, &col_cnt, &col_buf, &xs, &xr, &xc, &taken,
+                      &gather_send, &gather_recv, &misc, &ubuf, &done, &scnt};
         for (Buf *b : all) b->release();
         if (h_uncert) cudaFreeHost(h_uncert);
         if (h_pack) cudaFreeHost(h_pack);
@@ -273,7 +270,6 @@ static int ws_prepare(vm_store *s)
     ENS(w.q_f32, (size_t)MAXQ * s->ld * 4);
     ENS(w.q_bf16, (size_t)2 * MAXQ * s->ld * 2);  // hi terms, then lo terms (split query)
     ENS(w.cand, (size_t)lists * MAXQ * (MAXK > SCAN_SLAB ? MAXK : SCAN_SLAB) * 8);  // per-CTA lists / dumped tiles / slabs
-    ENS(w.merged, (size_t)MAXQ * MAXK * 8);
     ENS(w.o_idx, result_bytes(MAXQ, MAXK) + 64);
     ENS(w.flags, (size_t)(MAXQ + 2) * 4);
     // per-CTA maxima [256][64] + published per-query bounds [64] + their counter [64] + union-buffer counters [64] (scan_tc.cu);
@@ -282,7 +278,6 @@ static int ws_prepare(vm_store *s)
     ENS(w.ubuf, (size_t)MAXQ * SCAN_UNION_CAP * 8);
     ENS(w.done, 64);
     ENS(w.scnt, (size_t)256 * MAXQ * 4);
-    ENS(w.sel_inc, (size_t)MAXQ * 4);
     VM_CUDA_CHECK(cudaMemset(w.done.p, 0, 64));
     ENS(w.col_thr, (size_t)MAXQ * 4);
     ENS(w.col_cnt, (size_t)MAXQ * 4);
@@ -861,7 +856,7 @@ static int topk_batch(const TopkCall &c)
 
     int32_t *flags = (int32_t *)w.flags.p;
     int32_t *uncert = flags + c.nq;  // counter sits right after the nq flags (zeroed by the normalise kernel)
-    RescoreArgs rs{(const uint64_t *)w.merged.p, kp, s->exact_rows(), s->inv_norms, s->exact_dtype(), s->ld, s->dim, s->size, q_dev,
+    RescoreArgs rs{kp, s->exact_rows(), s->inv_norms, s->exact_dtype(), s->ld, s->dim, s->size, q_dev,
                    c.q_dtype, c.nq, eps, c.sum_mode, fin, flags, uncert, s->extreme,
                    kernel == 2 ? (float *)w.col_thr.p : nullptr, s->cum};
     // where the candidates are: the union buffer of the tcgen05 scan (complete band), its dumped tiles (every row),
@@ -873,13 +868,6 @@ static int topk_batch(const TopkCall &c)
         sel.seed_tab = a.ctas <= 256 ? (const uint32_t *)w.seed.p : nullptr; sel.nq_pad = nq_pad; sel.ksel = c.k; sel.band = a.band;
     } else { sel.cand = a.cand; sel.lists = a.ctas; sel.list_len = a.dump ? SCAN_DUMP_TILE : kp; sel.complete = a.dump ? 1 : 0; }
     rc = k_select_rescore(sel, rs, st, pdl);   // fused selection + exact rescoring + band settlement
-    if (rc == VM_ERR_UNSUPPORTED && !a.dump) {  // rows too large for shared memory: two kernels
-        if (union_src) rc = k_slab_top(sel, c.nq, kp, (uint64_t *)w.merged.p, (int *)w.sel_inc.p, st);
-        else rc = k_merge_candidates(a.cand, a.ctas, c.nq, kp, (uint64_t *)w.merged.p, st);
-        if (rc != VM_OK) return rc;
-        rc = k_rescore(rs, st, union_src ? (const int *)w.sel_inc.p : nullptr);
-        ++launches;
-    }
     if (rc != VM_OK) return rc;
     launches += 1;
 

@@ -281,7 +281,6 @@ struct FinalizeArgs {
     int32_t *out_count;  // [nq]
 };
 struct RescoreArgs {
-    const uint64_t *merged;
     int kp;
     const void *rows;
     const float *inv_norms;

@@ -1,4 +1,4 @@
-// select.cu -- everything after the streaming scan: candidate merge, binary64 rescoring in the
+// select.cu -- everything after the streaming scan: candidate selection, binary64 rescoring in the
 // reference's summation order + certification, the always-exact binary64 scan used for
 // uncertified queries, the cross-shard merge and the cross-query max-by-id merge.
 #include "common.cuh"
@@ -8,20 +8,14 @@
 namespace vm {
 
 // =========================================================================================
-// 1. merge per-CTA candidate sets -> the kp best keys per query
+// 1. fused candidate selection + exact rescoring + band settlement (ONE launch)
 // =========================================================================================
-// cand [lists][nq][kp] -> merged [nq][kp]: the kp largest keys in ARBITRARY order except that
-// slot kp-1 holds the smallest of them (the "worst candidate" the certification needs); unused
-// slots are 0.  One CTA per query.  Keys are unique, so an MSB-first radix select (8 passes of
-// 8 bits, shared-memory histogram + one warp scanning the 256 bins) yields the exact kp-th
-// largest key T; every key >= T is then emitted.  O(n) work instead of kp block-wide arg-max
-// rounds.
-static constexpr int MERGE_THREADS = 512;
+static constexpr int SR_THREADS = 512;
 static constexpr int MERGE_SURV = 1024;  // survivors ranked directly
 
-// Exact kp-th largest key of skeys[0..total) by MSB-first radix select (8 passes x 8 bits).
-// Block-wide; returns the same value in every thread.  Used when the cheap bound below does not
-// thin the keys enough (heavily duplicated scores).
+// Exact kp-th largest key of skeys[0..total) by MSB-first radix select (8 passes x 8 bits, shared-memory histogram + one
+// warp scanning the 256 bins).  Block-wide; returns the same value in every thread.  Used when the cheap bound of the
+// selection does not thin the keys enough (heavily duplicated scores, few lists, a large union).
 __device__ uint64_t radix_select_kth(const uint64_t *skeys, int total, int kp, int *hist, int *s_bin, int *s_need)
 {
     const int tid = threadIdx.x, lane = tid & 31;
@@ -32,7 +26,7 @@ __device__ uint64_t radix_select_kth(const uint64_t *skeys, int total, int kp, i
         const uint64_t hmask = pass == 0 ? 0ull : (~0ull << (shift + 8));
         if (tid < 256) hist[tid] = 0;
         __syncthreads();
-        for (int e = tid; e < total; e += MERGE_THREADS) {
+        for (int e = tid; e < total; e += SR_THREADS) {
             const uint64_t k = skeys[e];
             const bool act = k != 0 && (k & hmask) == prefix;
             const int bin = act ? (int)((k >> shift) & 0xFF) : -1;
@@ -67,150 +61,9 @@ __device__ uint64_t radix_select_kth(const uint64_t *skeys, int total, int kp, i
     return prefix;
 }
 
-// One CTA per query.
-//  1. every list's maximum score is found by one warp (32-bit REDUX); the kp-th largest of those
-//     maxima, L, is a lower bound on the kp-th largest key (kp different lists reach it);
-//  2. keys with score >= L ("survivors", typically ~kp..2kp of the lists*kp keys) are compacted;
-//  3. survivors are ranked against each other and written in descending order, so slot kp-1 is
-//     the worst candidate the certification needs.
-// Falls back to the exact radix select when fewer than kp lists are populated or more than
-// MERGE_SURV keys survive.
-__global__ void __launch_bounds__(MERGE_THREADS) merge_candidates_kernel(const uint64_t *__restrict__ cand, int lists, int nq,
-                                                                       int kp, uint64_t *__restrict__ merged)
-{
-    extern __shared__ uint64_t skeys[];  // [lists*kp] then [lists] list maxima (u32)
-    __shared__ uint64_t surv[MERGE_SURV];
-    __shared__ int hist[256];
-    __shared__ int s_bin, s_need, s_m, s_nz;
-    __shared__ uint32_t s_L;
-    const int q = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int total = lists * kp;
-    uint32_t *lmax = reinterpret_cast<uint32_t *>(skeys + total);
-    if (tid == 0) { s_m = 0; s_nz = 0; }
-    __syncthreads();
-    int nz = 0;
-#pragma unroll 4
-    for (int e = tid; e < total; e += MERGE_THREADS) {
-        int l = e / kp, j = e - l * kp;
-        uint64_t k = cand[((int64_t)l * nq + q) * kp + j];
-        skeys[e] = k;
-        nz += k != 0;
-    }
-    if (nz) atomicAdd(&s_nz, nz);
-    __syncthreads();
-    const int nonzero = s_nz;
-    uint64_t T = 1;  // smallest real key is > 0: T = 1 selects every non-empty slot
-    bool ranked_path = false;
-    if (nonzero >= kp) {
-        if (lists >= kp) {
-            // 1. per-list maximum score (high word of the key)
-            for (int l = warp; l < lists; l += MERGE_THREADS / 32) {
-                uint32_t m = 0;
-                for (int j = lane; j < kp; j += 32) m = max(m, (uint32_t)(skeys[l * kp + j] >> 32));
-                m = __reduce_max_sync(0xffffffffu, m);
-                if (lane == 0) lmax[l] = m;
-            }
-            __syncthreads();
-            if (warp == 0) {
-                // kp-th largest of the list maxima: bitwise radix select with warp reductions
-                uint32_t prefix = 0;
-                int need = kp;
-                for (int bit = 31; bit >= 0; --bit) {
-                    const uint32_t hi = bit == 31 ? 0u : (0xFFFFFFFFu << (bit + 1));
-                    int cnt = 0;
-                    for (int l = lane; l < lists; l += 32) cnt += ((lmax[l] & hi) == prefix && ((lmax[l] >> bit) & 1u)) ? 1 : 0;
-                    const int tot = __reduce_add_sync(0xffffffffu, cnt);
-                    if (tot >= need) prefix |= 1u << bit;
-                    else need -= tot;
-                }
-                if (lane == 0) s_L = prefix;
-            }
-            __syncthreads();
-            const uint32_t Lb = s_L;
-            if (Lb != 0) {
-                // 2. compact the survivors
-                for (int e = tid; e < total; e += MERGE_THREADS) {
-                    const uint64_t k = skeys[e];
-                    if ((uint32_t)(k >> 32) >= Lb && k != 0) {
-                        const int p = atomicAdd(&s_m, 1);
-                        if (p < MERGE_SURV) surv[p] = k;
-                    }
-                }
-                __syncthreads();
-                const int m = s_m;
-                if (m >= kp && m <= MERGE_SURV) {
-                    // 3. rank survivors (keys are unique) and emit the kp largest in descending order
-                    for (int e = tid; e < m; e += MERGE_THREADS) {
-                        const uint64_t k = surv[e];
-                        int rank = 0;
-                        for (int i = 0; i < m; ++i) rank += surv[i] > k ? 1 : 0;
-                        if (rank < kp) merged[(int64_t)q * kp + rank] = k;
-                    }
-                    ranked_path = true;
-                }
-            }
-        }
-        if (!ranked_path) {
-            __syncthreads();
-            T = radix_select_kth(skeys, total, kp, hist, &s_bin, &s_need);
-        }
-    }
-    if (ranked_path) return;  // uniform across the block
-    if (tid == 0) s_m = 0;
-    __syncthreads();
-    for (int e = tid; e < total; e += MERGE_THREADS) {
-        const uint64_t k = skeys[e];
-        if (k >= T && k != 0) {
-            if (nonzero >= kp && k == T) merged[(int64_t)q * kp + kp - 1] = k;  // the worst candidate
-            else merged[(int64_t)q * kp + atomicAdd(&s_m, 1)] = k;
-        }
-    }
-    __syncthreads();
-    const int filled = s_m;
-    const int last = nonzero >= kp ? kp - 1 : kp;
-    for (int e = filled + tid; e < last; e += MERGE_THREADS) merged[(int64_t)q * kp + e] = 0;
-}
-
-// =========================================================================================
-// 2. exact binary64 rescoring + sort + certification
-// =========================================================================================
-
 __device__ __forceinline__ double convert_score(double c, int score_mode)
 {
     return score_mode == VM_SCORE_NEO4J ? __ddiv_rn(__dadd_rn(1.0, c), 2.0) : c;
-}
-
-// Reference cosine on (query, row): pre_llm_injector.py:374-388 in binary64, products and sums
-// in index order.  Rows are read with their stored dtype; `dim` real columns only.
-template <bool NEUMAIER, typename T>
-__device__ double exact_cosine(const void *q, int q_dtype, int64_t qoff, const T *row, int dim)
-{
-    RefSum dot, qq, rr;
-    dot.init(); qq.init(); rr.init();
-    for (int i = 0; i < dim; ++i) {
-        double x = load_as_double(q, q_dtype, qoff + i);
-        double y = load_elem(row, i);
-        dot.add<NEUMAIER>(__dmul_rn(x, y));
-        qq.add<NEUMAIER>(__dmul_rn(x, x));
-        rr.add<NEUMAIER>(__dmul_rn(y, y));
-    }
-    double n1 = __dsqrt_rn(qq.result<NEUMAIER>());
-    double n2 = __dsqrt_rn(rr.result<NEUMAIER>());
-    if (n1 == 0.0 || n2 == 0.0) return 0.0;
-    return __ddiv_rn(dot.result<NEUMAIER>(), __dmul_rn(n1, n2));
-}
-
-// Same, with the query already staged as doubles in shared memory.
-template <bool NEUMAIER, typename T>
-__device__ double exact_cosine_sq(const double *sq, double n1, const T *row, int dim)
-{
-    RefSum dot, rr;
-    dot.init(); rr.init();
-    ref_sum_range<NEUMAIER>(dot, 0, dim, [&](int i) { return __dmul_rn(sq[i], load_elem(row, i)); });
-    ref_sum_range<NEUMAIER>(rr, 0, dim, [&](int i) { const double y = load_elem(row, i); return __dmul_rn(y, y); });
-    double n2 = __dsqrt_rn(rr.result<NEUMAIER>());
-    if (n1 == 0.0 || n2 == 0.0) return 0.0;
-    return __ddiv_rn(dot.result<NEUMAIER>(), __dmul_rn(n1, n2));
 }
 
 // (score desc, row asc) strict order
@@ -219,179 +72,6 @@ __device__ __forceinline__ bool better(double sa, uint32_t ra, double sb, uint32
     return sa > sb || (sa == sb && ra < rb);
 }
 
-// One CTA per query.  The reference formula needs three sequential binary64 sums per
-// (query, candidate): dot, ||q||^2 and ||row||^2.  Each is an independent chain, so they are
-// spread over threads as TASKS -- task t < kp: dot of candidate t; kp <= t < 2kp: ||row||^2 of
-// candidate t-kp; t == 2kp: ||q||^2 -- and every chain runs in index order (bit-identical to
-// CPython).  Query and candidate rows are staged through shared memory as doubles in column
-// chunks (coalesced loads; odd row pitch -> conflict-free per-thread walks).
-// eps: bound on |approximate cosine - exact cosine| of the scan that produced the candidates.
-static constexpr int RS_THREADS = 256;  // >= 2*64 + 1 tasks; the extra threads help staging
-static constexpr int RS_SMEM_ROW_BYTES = 96 * 1024;
-
-// 16-byte global load of 4 (fp32) / 8 (bf16) consecutive row elements -> floats
-__device__ __forceinline__ void load_vec16(const float *p, float *o)
-{
-    const float4 t = *reinterpret_cast<const float4 *>(p);
-    o[0] = t.x; o[1] = t.y; o[2] = t.z; o[3] = t.w;
-}
-__device__ __forceinline__ void load_vec16(const __nv_bfloat16 *p, float *o)
-{
-    const uint4 u = *reinterpret_cast<const uint4 *>(p);
-    o[0] = __uint_as_float(u.x << 16); o[1] = __uint_as_float(u.x & 0xffff0000u);
-    o[2] = __uint_as_float(u.y << 16); o[3] = __uint_as_float(u.y & 0xffff0000u);
-    o[4] = __uint_as_float(u.z << 16); o[5] = __uint_as_float(u.z & 0xffff0000u);
-    o[6] = __uint_as_float(u.w << 16); o[7] = __uint_as_float(u.w & 0xffff0000u);
-}
-
-__device__ __forceinline__ void load_vec16(const double *p, double *o)
-{
-    const double2 t = *reinterpret_cast<const double2 *>(p);
-    o[0] = t.x; o[1] = t.y;
-}
-// what a staged row element is held as in shared memory: float is exact for fp32 / bf16 rows, binary64 rows stay binary64
-template <typename T> struct StageOf { using type = float; };
-template <> struct StageOf<double> { using type = double; };
-
-template <bool NEUMAIER, typename T>
-__global__ void __launch_bounds__(RS_THREADS, 1) rescore_kernel(const uint64_t *__restrict__ merged, int kp, const T *__restrict__ rows,
-                                                            const float *__restrict__ inv_norms, int ld, int dim, int64_t n_rows,
-                                                            const void *__restrict__ queries, int q_dtype, double eps,
-                                                            FinalizeArgs f, int32_t *__restrict__ flags,
-                                                            int32_t *__restrict__ uncertified_count, int chunk,
-                                                            const int *__restrict__ extreme, float *__restrict__ collect_thr,
-                                                            unsigned long long *__restrict__ cum, const int *__restrict__ incomplete)
-{
-    constexpr int VEC = 16 / (int)sizeof(T);      // elements per 16-byte load
-    extern __shared__ double rs_smem[];
-    double *sq = rs_smem;                          // [chunk] query as doubles
-    using S = typename StageOf<T>::type;
-    S *srow = reinterpret_cast<S *>(rs_smem + chunk);  // [kp][chunk + 1] candidate rows (odd pitch)
-    const int pitch = chunk + 1;
-    __shared__ double s_dot[64], s_rr[64], s_qq;
-    __shared__ double s_score[64];
-    __shared__ uint32_t s_row[64];
-    __shared__ int s_valid[64];
-    __shared__ int s_cnt;
-    const int q = blockIdx.x, j = threadIdx.x;
-    if (j == 0) s_cnt = 0;
-    if (j < 64) {
-        uint64_t key = j < kp ? merged[(int64_t)q * kp + j] : 0;
-        s_valid[j] = key != 0;
-        s_row[j] = key != 0 ? key_row(key) : 0;
-    }
-    __syncthreads();
-    // task decode
-    const int kind = j < kp ? 0 : (j < 2 * kp ? 1 : (j == 2 * kp ? 2 : 3));
-    const int cand = kind == 0 ? j : (kind == 1 ? j - kp : 0);
-    const bool active = kind == 2 || (kind < 2 && s_valid[cand]);
-    RefSum acc;
-    acc.init();
-    for (int c0 = 0; c0 < dim; c0 += chunk) {
-        const int len = min(chunk, dim - c0);          // real columns in this chunk
-        const int vlen = (min(chunk, ld - c0) + VEC - 1) / VEC;  // 16-byte groups (rows are zero padded to ld)
-        for (int i = j; i < len; i += RS_THREADS) sq[i] = load_as_double(queries, q_dtype, (int64_t)q * dim + c0 + i);
-        // stage the candidate rows: batches of 4 independent 16-byte loads per thread
-        const int groups = kp * vlen;
-        for (int g0 = j; g0 < groups; g0 += 4 * RS_THREADS) {
-            S buf[4][VEC];
-            int rr_[4], cc_[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int g = g0 + u * RS_THREADS;
-                rr_[u] = g < groups ? g / vlen : -1;
-                cc_[u] = g < groups ? (g - rr_[u] * vlen) * VEC : 0;
-                if (rr_[u] >= 0 && s_valid[rr_[u]]) load_vec16(rows + (int64_t)s_row[rr_[u]] * ld + c0 + cc_[u], buf[u]);
-                else
-#pragma unroll
-                    for (int x = 0; x < VEC; ++x) buf[u][x] = (S)0;
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u)
-                if (rr_[u] >= 0)
-#pragma unroll
-                    for (int x = 0; x < VEC; ++x)
-                        if (cc_[u] + x < chunk) srow[rr_[u] * pitch + cc_[u] + x] = buf[u][x];
-        }
-        __syncthreads();
-        if (active) {
-            const S *mine = srow + cand * pitch;
-            if (kind == 0)
-                ref_sum_range<NEUMAIER>(acc, 0, len, [&](int i) { return __dmul_rn(sq[i], (double)mine[i]); });
-            else if (kind == 1)
-                ref_sum_range<NEUMAIER>(acc, 0, len, [&](int i) { const double y = (double)mine[i]; return __dmul_rn(y, y); });
-            else
-                ref_sum_range<NEUMAIER>(acc, 0, len, [&](int i) { const double x = sq[i]; return __dmul_rn(x, x); });
-        }
-        __syncthreads();
-    }
-    if (active) {
-        const double r = acc.result<NEUMAIER>();
-        if (kind == 0) s_dot[cand] = r;
-        else if (kind == 1) s_rr[cand] = r;
-        else s_qq = r;
-    }
-    __syncthreads();
-    const bool valid = j < 64 && s_valid[j];
-    double sc = 0.0;
-    const uint32_t row = j < 64 ? s_row[j] : 0;
-    if (valid) {
-        const double n1 = __dsqrt_rn(s_qq);
-        const double n2 = __dsqrt_rn(s_rr[j]);
-        sc = (n1 == 0.0 || n2 == 0.0) ? 0.0 : __ddiv_rn(s_dot[j], __dmul_rn(n1, n2));
-    }
-    if (j < 64) s_score[j] = sc;
-    __syncthreads();
-    int ncand = 0;
-    for (int i = 0; i < 64; ++i) ncand += s_valid[i];
-    // rank among valid candidates
-    int rank = 0;
-    if (valid)
-        for (int i = 0; i < 64; ++i)
-            if (s_valid[i] && i != j && better(s_score[i], s_row[i], sc, row)) ++rank;
-    double outv = convert_score(sc, f.score_mode);
-    bool emit = valid && rank < f.k && outv > f.min_score;
-    if (emit) {
-        f.out_idx[(int64_t)q * f.k + rank] = (int64_t)row + f.row_offset;
-        f.out_score[(int64_t)q * f.k + rank] = outv;
-        atomicAdd(&s_cnt, 1);
-    }
-    __syncthreads();
-    // certification: every non-candidate row r has approx(r) <= approx(worst candidate), hence
-    // exact(r) <= approx_worst + eps; certified iff that is strictly below the k-th exact score.
-    // Fewer than kp candidates means every scorable row of the shard is already a candidate.
-    // (merge_candidates_kernel puts the worst candidate in slot kp-1.)
-    if (valid && rank == min(f.k, ncand) - 1) {
-        bool cert = true;
-        if (ncand >= kp && (int64_t)ncand < n_rows) {
-            float worst = key_score(merged[(int64_t)q * kp + kp - 1]);
-            cert = ((double)worst + eps) < sc;
-        }
-        if (incomplete && incomplete[q]) cert = false;  // the slabs / spill buffer this list was taken from overflowed: rows are missing
-        // flag 1: a collect pass (all rows within 2 eps of this score) can settle the query;
-        // flag 2: the error bound does not hold for this store -> binary64 scan of every row
-        const bool bound_ok = !(extreme && *extreme != 0);
-        if (!bound_ok && (int64_t)ncand < n_rows) cert = false;
-        flags[q] = cert ? 0 : (bound_ok ? 1 : 2);
-        if (collect_thr) {
-            float t = (float)(sc - 2.0 * eps);
-            t = nextafterf(nextafterf(t, -INFINITY), -INFINITY);  // the cast may have rounded up
-            collect_thr[q] = (!cert && bound_ok) ? t : INFINITY;
-        }
-        if (!cert) { atomicAdd(uncertified_count, 1); if (cum) atomicAdd(cum, 1ull); }
-    }
-    if (ncand == 0 && j == 0) { flags[q] = 0; if (collect_thr) collect_thr[q] = INFINITY; }
-    if (j == 0) f.out_count[q] = s_cnt;
-    int cnt = s_cnt;
-    for (int t = cnt + j; t < f.k; t += RS_THREADS) {
-        f.out_idx[(int64_t)q * f.k + t] = -1;
-        f.out_score[(int64_t)q * f.k + t] = 0.0;
-    }
-}
-
-// =========================================================================================
-// 2b. fused candidate selection + exact rescoring + band settlement (the normal path: ONE launch)
-// =========================================================================================
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc)
 {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
@@ -399,48 +79,11 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc)
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-static constexpr int SR_THREADS = 512;
 // Rows of one query's near-tie band the rescoring kernel settles itself: as many as shared memory leaves room for
 // (12 bytes each), between BAND_CAP_MIN and BAND_CAP_MAX.  Settling 2048 rows costs ~0.3 ms for the batch (64 staged
 // sub-batches per query, the queries in parallel) and no extra pass over the store; bands of up to 4096 rows are left
 // to the collect pass (a second streaming scan + its own rescoring), anything larger to the binary64 scan.
 static constexpr int BAND_CAP_MIN = 1024, BAND_CAP_MAX = 2048;
-
-// Exact scores of m gathered rows straight from global memory (block-wide; the collect pass, whose row sets do not fit
-// shared memory).  The rows sit in DRAM (the scan streams them through L2 with evict-first), so all their 128-byte lines
-// are first pulled into L2 by the whole block at once -- a thread walking its row would otherwise pay one serial DRAM
-// miss per line.  Then 2m independent sequential chains (dot and ||row||^2 per row: the reference recurrences, in index
-// order) run on 2m threads.  s_sc / s_rr / s_row: [m]; on return s_sc holds the reference scores.
-template <bool NEUMAIER, typename T, int THREADS>
-__device__ void band_score_global(const T *__restrict__ rows, int ld, int dim, const double *sq, double n1, int m, double *s_sc, double *s_rr,
-                                  const uint32_t *s_row)
-{
-    const int tid = threadIdx.x;
-    const int lines = (ld * (int)sizeof(T) + 127) / 128;
-    for (int e = tid; e < m * lines; e += THREADS) {
-        const int r = e / lines, l = e - r * lines;
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char *>(rows + (int64_t)s_row[r] * ld) + (size_t)l * 128));
-    }
-    for (int t = tid; t < 2 * m; t += THREADS) {
-        const int e = t >> 1;
-        const T *row = rows + (int64_t)s_row[e] * ld;
-        RefSum acc;
-        acc.init();
-        if (t & 1) {
-            ref_sum_range<NEUMAIER>(acc, 0, dim, [&](int i) { const double y = load_elem(row, i); return __dmul_rn(y, y); });
-            s_rr[e] = acc.result<NEUMAIER>();
-        } else {
-            ref_sum_range<NEUMAIER>(acc, 0, dim, [&](int i) { return __dmul_rn(sq[i], load_elem(row, i)); });
-            s_sc[e] = acc.result<NEUMAIER>();
-        }
-    }
-    __syncthreads();
-    for (int e = tid; e < m; e += THREADS) {
-        const double n2 = __dsqrt_rn(s_rr[e]);
-        s_sc[e] = (n1 == 0.0 || n2 == 0.0) ? 0.0 : __ddiv_rn(s_sc[e], __dmul_rn(n1, n2));
-    }
-    __syncthreads();
-}
 
 // Exact top-k among m rows with reference scores s_sc (block-wide): every row is ranked by counting the rows that beat it
 // (score desc, row asc: rows are distinct, so ranks are) and the first k are emitted.  Returns the number of entries
@@ -477,46 +120,56 @@ __device__ int band_emit(int m, const double *s_sc, const uint32_t *s_row, int *
 
 static constexpr uint32_t NO_ROW = 0xFFFFFFFFu;
 
-// Stages up to kp rows (ids in s_rid[0, kp), NO_ROW = none) in shared memory with cp.async (16-byte, L2-cached, three
-// column chunks; coalesced -- 32 threads each walking their own row in global memory would serialise in the load unit,
-// one tag lookup per row per instruction) and runs the reference recurrences as independent sequential chains, chunk c
-// overlapping the loads of chunk c+1: thread j < kp: dot(query, row j); kp <= j < 2 kp: ||row j-kp||^2; j == 2 kp and
-// s_qq != NULL: ||query||^2.  Results -> s_dot / s_rr / *s_qq.  Block-wide; ends with a barrier.
+// Stages up to kp rows (ids in s_rid[0, kp), NO_ROW = none) in shared memory with cp.async (16-byte, L2-cached;
+// coalesced -- 32 threads each walking their own row in global memory would serialise in the load unit, one tag lookup per
+// row per instruction) and runs the reference recurrences as independent sequential chains: thread j < kp: dot(query,
+// row j); kp <= j < 2 kp: ||row j-kp||^2; j == 2 kp and s_qq != NULL: ||query||^2.  Results -> s_dot / s_rr / *s_qq.
+// The rows are staged in `chunks` (>= 3) column chunks -- chunk c: the 16-byte groups [c*gpr/chunks, (c+1)*gpr/chunks)
+// of every row -- through a ring of three slots: slot b starts at group b*win/3 of a staged row of `pitch` = 16*(win+1)
+// bytes.  The chains run over chunk c while chunks c+1 and c+2 load; then chunk c+3 goes into the slot chunk c frees.
+// Three chunks with win = gpr are whole rows, every chunk in its own columns.  Each chain still runs over the columns in
+// index order.  Block-wide; ends with a barrier.
 template <bool NEUMAIER, typename T, int THREADS>
 __device__ __forceinline__ void stage_and_chain(const T *__restrict__ rows, int ld, int dim, int kp, const uint32_t *s_rid,
-                                                unsigned char *srow, int pitch, const double *sq, double *s_dot, double *s_rr, double *s_qq)
+                                                unsigned char *srow, int pitch, int chunks, const double *sq, double *s_dot,
+                                                double *s_rr, double *s_qq)
 {
     const int tid = threadIdx.x, j = tid;
     const int gpr = ld * (int)sizeof(T) / 16;                 // 16-byte groups per row
-    const int c1 = gpr / 3, c2 = 2 * gpr / 3;                 // chunk boundaries (in groups)
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        const int g_lo = c == 0 ? 0 : (c == 1 ? c1 : c2), g_hi = c == 0 ? c1 : (c == 1 ? c2 : gpr);
-        const int w = g_hi - g_lo;
+    const int win = pitch / 16 - 1;                           // 16-byte groups per staged row
+    auto g_lo = [&](int c) { return c * gpr / chunks; };      // first group of chunk c
+    auto slot = [&](int c) { return (c % 3) * win / 3; };     // first staged group of chunk c's slot
+    auto issue = [&](int c) {
+        const int lo = g_lo(c), w = g_lo(c + 1) - lo, base = slot(c);
         for (int e = tid; e < kp * w; e += THREADS) {
-            const int r = e / w, g = g_lo + (e - r * w);
+            const int r = e / w, g = e - r * w;
             const uint32_t rid = s_rid[r];
             if (rid != NO_ROW)
-                cp_async16(srow + (size_t)r * pitch + (size_t)g * 16,
-                           reinterpret_cast<const unsigned char *>(rows + (int64_t)rid * ld) + (size_t)g * 16);
+                cp_async16(srow + (size_t)r * pitch + (size_t)(base + g) * 16,
+                           reinterpret_cast<const unsigned char *>(rows + (int64_t)rid * ld) + (size_t)(lo + g) * 16);
         }
         cp_async_commit();
-    }
+    };
+    issue(0);
+    issue(1);
+    issue(2);
     const int kind = j < kp ? 0 : (j < 2 * kp ? 1 : ((j == 2 * kp && s_qq != nullptr) ? 2 : 3));
     const int cidx = kind == 0 ? j : (kind == 1 ? j - kp : 0);
     const bool active = kind == 2 || (kind < 2 && s_rid[cidx] != NO_ROW);
-    const T *mine = reinterpret_cast<const T *>(srow + (size_t)cidx * pitch);
     constexpr int EPG = 16 / (int)sizeof(T);                  // elements per 16-byte group
     RefSum acc;
     acc.init();
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        if (c == 0) cp_async_wait<2>();
-        else if (c == 1) cp_async_wait<1>();
+    for (int c = 0, lo = 0; c < chunks; ++c) {
+        // groups 0..c must have landed; chunks c+1 and c+2, where they exist, may still be in flight
+        if (c + 2 < chunks) cp_async_wait<2>();
+        else if (c + 1 < chunks) cp_async_wait<1>();
         else cp_async_wait<0>();
         __syncthreads();
-        const int g_lo = c == 0 ? 0 : (c == 1 ? c1 : c2), g_hi = c == 0 ? c1 : (c == 1 ? c2 : gpr);
-        const int i_lo = g_lo * EPG, i_hi = min(g_hi * EPG, dim);
+        const int hi = g_lo(c + 1);
+        const int i_lo = lo * EPG, i_hi = min(hi * EPG, dim);
+        // column i of this chunk is mine[i]
+        const T *mine = reinterpret_cast<const T *>(srow + (size_t)cidx * pitch + (ptrdiff_t)(slot(c) - lo) * 16);
+        lo = hi;
         if (active) {
             if (kind == 0)
                 ref_sum_range<NEUMAIER>(acc, i_lo, i_hi, [&](int i) { return __dmul_rn(sq[i], load_elem(mine, i)); });
@@ -524,6 +177,10 @@ __device__ __forceinline__ void stage_and_chain(const T *__restrict__ rows, int 
                 ref_sum_range<NEUMAIER>(acc, i_lo, i_hi, [&](int i) { const double y = load_elem(mine, i); return __dmul_rn(y, y); });
             else
                 ref_sum_range<NEUMAIER>(acc, i_lo, i_hi, [&](int i) { const double x = sq[i]; return __dmul_rn(x, x); });
+        }
+        if (c + 3 < chunks) {
+            __syncthreads();  // every chain is done with chunk c's slot
+            issue(c + 3);
         }
     }
     if (active) {
@@ -553,6 +210,7 @@ struct SelectSrc {
     float band;
     int key_cap;           // keys one CTA stages in shared memory
     int band_cap;          // band rows one CTA can settle (shared-memory room, see BAND_CAP_MIN / MAX)
+    int pitch, chunks;     // staged-row window of stage_and_chain (stage_window)
 };
 
 // Slab mode: stages query q's keys in shared memory, filtered once more with the FINAL bound -- the k-th largest of the
@@ -614,47 +272,14 @@ __device__ int load_slab_keys(const SelectSrc &src, int q, int nq, uint64_t *ske
     return min(got, src.key_cap);
 }
 
-// Slab-mode form of the merge for rows too large for the fused kernel's shared memory: the query's filtered keys ->
-// its kp best in descending order, zero padded; incomplete[q] = keys were missing.  One CTA per query.
-__global__ void __launch_bounds__(SR_THREADS) slab_top_kernel(SelectSrc src, int nq, int kp, uint64_t *__restrict__ merged,
-                                                             int *__restrict__ incomplete)
-{
-    extern __shared__ __align__(16) unsigned char st_smem[];
-    uint64_t *skeys = reinterpret_cast<uint64_t *>(st_smem);  // [key_cap]
-    __shared__ int s_cnts[256];
-    __shared__ int s_total, s_bin, s_need, s_m;
-    __shared__ int hist[256];
-    __shared__ float s_bf;
-    const int q = blockIdx.x, tid = threadIdx.x;
-    bool inc = false;
-    const int total = load_slab_keys<SR_THREADS>(src, q, nq, skeys, s_cnts, &s_total, &s_bf, &inc);
-    for (int e = tid; e < kp; e += SR_THREADS) merged[(int64_t)q * kp + e] = 0;
-    if (tid == 0) { incomplete[q] = inc ? 1 : 0; s_m = 0; }
-    __syncthreads();
-    if (total <= MERGE_SURV) {
-        for (int e = tid; e < total; e += SR_THREADS) {
-            const uint64_t k = skeys[e];
-            int rank = 0;
-            for (int i = 0; i < total; ++i) rank += skeys[i] > k ? 1 : 0;
-            if (rank < kp) merged[(int64_t)q * kp + rank] = k;
-        }
-        return;
-    }
-    const uint64_t Tk = radix_select_kth(skeys, total, kp, hist, &s_bin, &s_need);
-    for (int e = tid; e < total; e += SR_THREADS) {
-        const uint64_t k = skeys[e];
-        if (k > Tk) merged[(int64_t)q * kp + atomicAdd(&s_m, 1)] = k;
-        else if (k == Tk) merged[(int64_t)q * kp + kp - 1] = k;  // the worst candidate goes last
-    }
-}
-
 // One CTA (512 threads) per query:
 //   A. the query's candidate keys are loaded into shared memory (union buffer: typically a few dozen keys; dumped
-//      tiles / per-CTA lists: thinned with the list-maxima bound, see merge_candidates_kernel) and the kp best by
-//      approximate score are ranked;
-//   B. their rows are pulled into shared memory with cp.async (16-byte, L2-cached) in three column chunks;
+//      tiles / per-CTA lists: thinned with a lower bound on the kp-th key, the kp-th largest of the lists' maxima)
+//      and the kp best by approximate score are ranked;
+//   B. their rows are pulled into shared memory with cp.async (16-byte, L2-cached) in column chunks, three slots of
+//      them in flight (stage_and_chain);
 //   C. the reference recurrences (dot per candidate, ||row||^2 per candidate, ||q||^2) run as independent
-//      sequential chains on 2kp+1 threads, chunk c overlapping the loads of chunk c+1;
+//      sequential chains on 2kp+1 threads, chunk c overlapping the loads of chunks c+1 and c+2;
 //   D. rank, emit, certify: with s_k the k-th exact score, only rows whose approximate score reaches s_k - eps can
 //      still matter.  When the source is complete they are all in shared memory already: if they are all among the
 //      rescored kp the list is final, otherwise
@@ -676,9 +301,9 @@ __global__ void __launch_bounds__(SR_THREADS, 1) select_rescore_kernel(SelectSrc
     uint64_t *skeys = reinterpret_cast<uint64_t *>(sr_smem);                       // [key_cap]
     uint32_t *lmax = reinterpret_cast<uint32_t *>(skeys + src.key_cap);            // [lists] (+pad)
     double *sq = reinterpret_cast<double *>(lmax + ((src.lists + 3) & ~3));        // [dim]
-    const int pitch = ld * (int)sizeof(T) + 16;                                    // bytes, 16-B aligned rows
+    const int pitch = src.pitch;                                                   // bytes, a multiple of 16
     unsigned char *srow = reinterpret_cast<unsigned char *>(sq + ((dim + 1) & ~1)); // [kp][pitch] staged rows
-    double *b_sc = reinterpret_cast<double *>(srow + (((size_t)kp * pitch + 15) & ~(size_t)15));  // [band_cap] band scores
+    double *b_sc = reinterpret_cast<double *>(srow + (size_t)kp * pitch);          // [band_cap] band scores
     uint32_t *b_row = reinterpret_cast<uint32_t *>(b_sc + src.band_cap);                       // [band_cap] band rows
     __shared__ uint64_t s_top[64];
     __shared__ uint32_t s_rid[64];
@@ -801,7 +426,7 @@ __global__ void __launch_bounds__(SR_THREADS, 1) select_rescore_kernel(SelectSrc
     const bool cand_valid = j < kp && mykey != 0;
     if (j < 64) s_rid[j] = cand_valid ? key_row(mykey) : NO_ROW;
     __syncthreads();
-    stage_and_chain<NEUMAIER, T, SR_THREADS>(rows, ld, dim, kp, s_rid, srow, pitch, sq, s_dot, s_rr, &s_qq);
+    stage_and_chain<NEUMAIER, T, SR_THREADS>(rows, ld, dim, kp, s_rid, srow, pitch, src.chunks, sq, s_dot, s_rr, &s_qq);
 
     // ---------------- D. rank, emit, certify ----------------
     double sc = 0.0;
@@ -902,7 +527,7 @@ __global__ void __launch_bounds__(SR_THREADS, 1) select_rescore_kernel(SelectSrc
             const int cnt = min(kp, band - b0);
             if (tid < 64) s_rid[tid] = tid < cnt ? b_row[b0 + tid] : NO_ROW;
             __syncthreads();
-            stage_and_chain<NEUMAIER, T, SR_THREADS>(rows, ld, dim, kp, s_rid, srow, pitch, sq, s_dot, s_rr, nullptr);
+            stage_and_chain<NEUMAIER, T, SR_THREADS>(rows, ld, dim, kp, s_rid, srow, pitch, src.chunks, sq, s_dot, s_rr, nullptr);
             if (tid < cnt) {
                 const double n2 = __dsqrt_rn(s_rr[tid]);
                 b_sc[b0 + tid] = (n1 == 0.0 || n2 == 0.0) ? 0.0 : __ddiv_rn(s_dot[tid], __dmul_rn(n1, n2));
@@ -937,30 +562,28 @@ __global__ void __launch_bounds__(SR_THREADS, 1) select_rescore_kernel(SelectSrc
 }
 
 // =========================================================================================
-// 2c. collect pass: exact top-k among the rows the second scan gathered for an uncertified query
+// 2. collect pass: exact top-k among the rows the second scan gathered for an uncertified query
 // =========================================================================================
 // One CTA (512 threads) per query with flag 1.  The collect scan stored every row whose approximate
 // score reached (exact k-th candidate score - 2 eps): that set contains the reference's top-k (a row
 // outside it is more than eps below the k-th candidate).  All gathered rows are scored with the
-// reference recurrence (band_score_global + band_emit) and the best k by (score desc, row asc) are emitted; the query's flag is
-// cleared.  If the buffer overflowed the flag becomes 2 and the binary64 scan of every row takes over.
+// reference recurrence (stage_and_chain, CR_ROWS rows at a time, then band_emit) and the best k by (score desc, row asc)
+// are emitted; the query's flag is cleared.  If the buffer overflowed the flag becomes 2 and the binary64 scan of every
+// row takes over.
 static constexpr int CR_THREADS = 512;
+static constexpr int CR_ROWS = 32;  // rows staged at a time
 template <bool NEUMAIER, typename T>
 __global__ void __launch_bounds__(CR_THREADS, 1) collect_rescore_kernel(const uint64_t *__restrict__ buf, const int *__restrict__ cnt, int cap,
                                                                        const T *__restrict__ rows, int ld, int dim,
                                                                        const void *__restrict__ queries, int q_dtype, FinalizeArgs f,
                                                                        int32_t *__restrict__ flags, int32_t *__restrict__ uncertified_count,
-                                                                       int nq, unsigned long long *__restrict__ cum, int stage_rows)
+                                                                       int nq, unsigned long long *__restrict__ cum, int pitch, int chunks)
 {
-    // stage_rows > 0: the gathered rows take the rescoring kernel's staged route (stage_and_chain), stage_rows at a time;
-    // 0 (rows too wide for shared memory): they are scored straight from global memory
     extern __shared__ __align__(16) unsigned char cr_smem[];
     double *sq = reinterpret_cast<double *>(cr_smem);               // [dim]
     double *s_sc = sq + ((dim + 1) & ~1);                           // [cap]
-    double *s_rr = s_sc + cap;                                      // [cap] (global route only)
-    uint32_t *s_row = reinterpret_cast<uint32_t *>(s_sc + (stage_rows > 0 ? cap : 2 * cap));     // [cap]
-    const int pitch = ld * (int)sizeof(T) + 16;
-    unsigned char *srow = reinterpret_cast<unsigned char *>(s_row + ((cap + 3) & ~3));  // [stage_rows][pitch] (staged route only)
+    uint32_t *s_row = reinterpret_cast<uint32_t *>(s_sc + cap);     // [cap]
+    unsigned char *srow = reinterpret_cast<unsigned char *>(s_row + ((cap + 3) & ~3));  // [CR_ROWS][pitch] staged rows
     __shared__ double s_n1;
     __shared__ int s_out;
     __shared__ uint32_t s_rid[64];
@@ -981,21 +604,17 @@ __global__ void __launch_bounds__(CR_THREADS, 1) collect_rescore_kernel(const ui
         s_n1 = __dsqrt_rn(qq.result<NEUMAIER>());
     }
     __syncthreads();
-    if (stage_rows > 0) {
-        const double n1 = s_n1;
-        for (int b0 = 0; b0 < m; b0 += stage_rows) {
-            const int c = min(stage_rows, m - b0);
-            if (tid < 64) s_rid[tid] = tid < c ? s_row[b0 + tid] : NO_ROW;
-            __syncthreads();
-            stage_and_chain<NEUMAIER, T, CR_THREADS>(rows, ld, dim, stage_rows, s_rid, srow, pitch, sq, s_dot, s_r2, nullptr);
-            if (tid < c) {
-                const double n2 = __dsqrt_rn(s_r2[tid]);
-                s_sc[b0 + tid] = (n1 == 0.0 || n2 == 0.0) ? 0.0 : __ddiv_rn(s_dot[tid], __dmul_rn(n1, n2));
-            }
-            __syncthreads();
+    const double n1 = s_n1;
+    for (int b0 = 0; b0 < m; b0 += CR_ROWS) {
+        const int c = min(CR_ROWS, m - b0);
+        if (tid < 64) s_rid[tid] = tid < c ? s_row[b0 + tid] : NO_ROW;
+        __syncthreads();
+        stage_and_chain<NEUMAIER, T, CR_THREADS>(rows, ld, dim, CR_ROWS, s_rid, srow, pitch, chunks, sq, s_dot, s_r2, nullptr);
+        if (tid < c) {
+            const double n2 = __dsqrt_rn(s_r2[tid]);
+            s_sc[b0 + tid] = (n1 == 0.0 || n2 == 0.0) ? 0.0 : __ddiv_rn(s_dot[tid], __dmul_rn(n1, n2));
         }
-    } else {
-        band_score_global<NEUMAIER, T, CR_THREADS>(rows, ld, dim, sq, s_n1, m, s_sc, s_rr, s_row);
+        __syncthreads();
     }
     band_emit<CR_THREADS>(m, s_sc, s_row, &s_out, f, q);
     if (tid == 0) {
@@ -1438,17 +1057,6 @@ __global__ void cosine_pairs_kernel(const void *__restrict__ a, const void *__re
 }
 
 // ---- host wrappers ---------------------------------------------------------------------
-int k_merge_candidates(const uint64_t *cand, int lists, int nq, int kp, uint64_t *merged, cudaStream_t st)
-{
-    size_t smem = (size_t)lists * kp * sizeof(uint64_t) + (size_t)lists * sizeof(uint32_t) + 16;
-    VM_CUDA_CHECK((max_smem_once<merge_candidates_kernel>(200 * 1024)));
-    VM_REQUIRE(smem <= 200 * 1024, VM_ERR_UNSUPPORTED, "candidate merge: %d lists x %d exceeds shared memory", lists, kp);
-    merge_candidates_kernel<<<nq, MERGE_THREADS, smem, st>>>(cand, lists, nq, kp, merged);
-    VM_CUDA_CHECK(cudaGetLastError());
-    return VM_OK;
-}
-
-
 // Calls f(neu) with neu a std::integral_constant<bool, Neumaier summation>, so f instantiates the matching
 // <NEUMAIER> kernel.
 template <typename F>
@@ -1467,53 +1075,47 @@ static int with_row_type(int dtype, int sum_mode, F &&f)
     return by_sum((__nv_bfloat16 *)nullptr);
 }
 
-int k_rescore(const RescoreArgs &a, cudaStream_t st, const int *incomplete)
+// The staged-row window of stage_and_chain for `rows` rows in `room` bytes of shared memory: whole rows in three chunks
+// when they fit (one 16-byte group of padding per row), else the fewest chunks whose three slots fit.  The windowed
+// pitch is an odd number of 16-byte groups, as whole fp32 / binary64 rows are, so that the chains, each walking its own
+// row at the same column, spread over the shared-memory banks.  chunks == 0: not even one group per slot fits.
+struct StageWindow { int pitch, chunks; };
+static StageWindow stage_window(int rows, int dtype, int ld, size_t room)
 {
-    // column chunk: whole rows when kp rows fit in RS_SMEM_ROW_BYTES, else a multiple of 8 columns
-    const int ssz = a.dtype == VM_F64 ? 8 : 4;  // staged element size (StageOf)
-    int chunk = RS_SMEM_ROW_BYTES / (ssz * a.kp) - 1;
-    chunk &= ~7;
-    if (chunk > a.ld) chunk = a.ld;
-    const size_t smem = (size_t)chunk * sizeof(double) + (size_t)a.kp * (chunk + 1) * ssz + 16;
-    return with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
-        using T = std::remove_pointer_t<decltype(tag)>;
-        constexpr bool NEU = decltype(neu)::value;
-        VM_CUDA_CHECK((max_smem_once<rescore_kernel<NEU, T>>(160 * 1024)));
-        rescore_kernel<NEU, T><<<a.nq, RS_THREADS, smem, st>>>(a.merged, a.kp, (const T *)a.rows, a.inv_norms, a.ld, a.dim,
-                                                               a.n_rows, a.queries, a.q_dtype, a.eps, a.fin, a.flags,
-                                                               a.uncertified_count, chunk, a.extreme, a.collect_thr, a.cum, incomplete);
-        VM_CUDA_CHECK(cudaGetLastError());
-        return VM_OK;
-    });
+    const int gpr = ld * (int)dtype_size(dtype) / 16;        // 16-byte groups per row
+    if ((size_t)rows * (gpr + 1) * 16 <= room) return {(gpr + 1) * 16, 3};
+    for (int chunks = 4; chunks <= gpr; ++chunks) {
+        const int s = (gpr + chunks - 1) / chunks;           // groups of the widest chunk
+        const int win = 3 * s + (s & 1);                     // three slots of >= s groups, win + 1 odd
+        if ((size_t)rows * (win + 1) * 16 <= room) return {(win + 1) * 16, chunks};
+    }
+    return {0, 0};
 }
 
-
-// Fused path when the candidate keys + kp whole rows fit in shared memory; otherwise the caller falls
-// back to k_merge_candidates + k_rescore.  Returns VM_ERR_UNSUPPORTED (without setting an error the
-// caller must report) when it does not apply.
+// Shared memory of select_rescore_kernel: keys, list maxima, query and the staged-row window, sized to leave room for at
+// least BAND_CAP_MIN band rows; then as many band rows (12 bytes each) as fit, up to BAND_CAP_MAX.  band_cap == 0: the
+// shape does not fit.
 static constexpr size_t SR_SMEM_LIMIT = 180 * 1024;
-// everything but the band scratch
-static size_t select_rescore_base_smem(int key_cap, int lists, int kp, int dtype, int dim, int ld)
+struct SelectLayout { StageWindow win; int band_cap; size_t smem; };
+static SelectLayout select_layout(int key_cap, int lists, int kp, int dtype, int dim, int ld)
 {
-    const int es = (int)dtype_size(dtype);
-    const size_t rows_area = (((size_t)kp * ((size_t)ld * es + 16) + 15) & ~(size_t)15) + 16;  // staged rows
-    return (size_t)key_cap * 8 + (size_t)((lists + 3) & ~3) * 4 + (size_t)((dim + 1) & ~1) * 8 + rows_area + 32;
-}
-// band rows that fit next to it (0: not even BAND_CAP_MIN)
-static int select_band_cap(int key_cap, int lists, int kp, int dtype, int dim, int ld)
-{
-    const size_t base = select_rescore_base_smem(key_cap, lists, kp, dtype, dim, ld);
-    if (base + (size_t)BAND_CAP_MIN * 12 > SR_SMEM_LIMIT) return 0;
-    size_t cap = (SR_SMEM_LIMIT - base) / 12;
-    cap &= ~(size_t)63;
-    if (cap > (size_t)BAND_CAP_MAX) cap = BAND_CAP_MAX;
-    return (int)cap;
+    const size_t fixed = (size_t)key_cap * 8 + (size_t)((lists + 3) & ~3) * 4 + (size_t)((dim + 1) & ~1) * 8 + 16 + 32;
+    const size_t need = fixed + (size_t)BAND_CAP_MIN * 12;
+    SelectLayout L{{0, 0}, 0, 0};
+    if (need > SR_SMEM_LIMIT) return L;
+    L.win = stage_window(kp, dtype, ld, SR_SMEM_LIMIT - need);
+    if (L.win.chunks == 0) return L;
+    const size_t base = fixed + (size_t)kp * L.win.pitch;
+    const size_t cap = ((SR_SMEM_LIMIT - base) / 12) & ~(size_t)63;
+    L.band_cap = (int)(cap < (size_t)BAND_CAP_MAX ? cap : (size_t)BAND_CAP_MAX);
+    L.smem = base + (size_t)L.band_cap * 12;
+    return L;
 }
 // lists == 0: slab mode (tcgen05 scan); else list mode with lists x list_len keys per query
 bool select_rescore_fits(int lists, int list_len, int kp, int dtype, int dim, int ld)
 {
     const int key_cap = lists > 0 ? lists * list_len : SELECT_KEY_CAP;
-    return select_band_cap(key_cap, lists, kp, dtype, dim, ld) >= BAND_CAP_MIN && kp <= 64 && 2 * kp + 1 <= SR_THREADS;
+    return select_layout(key_cap, lists, kp, dtype, dim, ld).band_cap >= BAND_CAP_MIN && kp <= 64 && 2 * kp + 1 <= SR_THREADS;
 }
 
 static SelectSrc make_src(const SelectArgs &sa)
@@ -1521,21 +1123,24 @@ static SelectSrc make_src(const SelectArgs &sa)
     const bool slab_mode = sa.slab != nullptr;
     const int lists = slab_mode ? 0 : sa.lists;
     return SelectSrc{sa.cand, lists, sa.list_len, sa.complete, sa.slab, sa.scnt, sa.ctas, sa.ubuf, sa.ucnt, sa.ucap, sa.seed_tab,
-                     sa.nq_pad, sa.ksel, sa.band, slab_mode ? SELECT_KEY_CAP : lists * sa.list_len, 0};
+                     sa.nq_pad, sa.ksel, sa.band, slab_mode ? SELECT_KEY_CAP : lists * sa.list_len, 0, 0, 0};
 }
 
 int k_select_rescore(const SelectArgs &sa, const RescoreArgs &a, cudaStream_t st, bool pdl)
 {
     SelectSrc src = make_src(sa);
     VM_REQUIRE(src.slab == nullptr || src.ctas <= 256, VM_ERR_UNSUPPORTED, "select: %d scan CTAs exceed 256", src.ctas);
-    if (!select_rescore_fits(src.lists, src.list_len, a.kp, a.dtype, a.dim, a.ld)) return VM_ERR_UNSUPPORTED;
-    src.band_cap = select_band_cap(src.key_cap, src.lists, a.kp, a.dtype, a.dim, a.ld);
-    const size_t smem = select_rescore_base_smem(src.key_cap, src.lists, a.kp, a.dtype, a.dim, a.ld) + (size_t)src.band_cap * 12;
+    VM_REQUIRE(select_rescore_fits(src.lists, src.list_len, a.kp, a.dtype, a.dim, a.ld), VM_ERR_UNSUPPORTED,
+               "select: %d keys and %d candidate rows of %d columns exceed shared memory", src.key_cap, a.kp, a.dim);
+    const SelectLayout L = select_layout(src.key_cap, src.lists, a.kp, a.dtype, a.dim, a.ld);
+    src.band_cap = L.band_cap;
+    src.pitch = L.win.pitch;
+    src.chunks = L.win.chunks;
     return with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
         using T = std::remove_pointer_t<decltype(tag)>;
         constexpr bool NEU = decltype(neu)::value;
         VM_CUDA_CHECK((max_smem_once<select_rescore_kernel<NEU, T>>(180 * 1024)));
-        VM_CUDA_CHECK(launch_pdl(select_rescore_kernel<NEU, T>, dim3(a.nq), dim3(SR_THREADS), smem, st, pdl, src, a.nq, a.kp,
+        VM_CUDA_CHECK(launch_pdl(select_rescore_kernel<NEU, T>, dim3(a.nq), dim3(SR_THREADS), L.smem, st, pdl, src, a.nq, a.kp,
                                  (const T *)a.rows, a.ld, a.dim, a.n_rows, a.queries, a.q_dtype, a.eps, a.fin, a.flags,
                                  a.uncertified_count, a.extreme, a.collect_thr, a.cum, a.inv_norms));
         VM_CUDA_CHECK(cudaGetLastError());
@@ -1543,30 +1148,21 @@ int k_select_rescore(const SelectArgs &sa, const RescoreArgs &a, cudaStream_t st
     });
 }
 
-// slab-mode selection alone (rows too large for the fused kernel): merged [nq][kp], incomplete [nq]
-int k_slab_top(const SelectArgs &sa, int nq, int kp, uint64_t *merged, int *incomplete, cudaStream_t st)
-{
-    const SelectSrc src = make_src(sa);
-    VM_REQUIRE(src.slab != nullptr && src.ctas <= 256, VM_ERR_UNSUPPORTED, "slab selection: bad source");
-    slab_top_kernel<<<nq, SR_THREADS, (size_t)src.key_cap * 8, st>>>(src, nq, kp, merged, incomplete);
-    VM_CUDA_CHECK(cudaGetLastError());
-    return VM_OK;
-}
-
 int k_collect_rescore(const uint64_t *buf, const int *cnt, int cap, const RescoreArgs &a, cudaStream_t st)
 {
-    // staged route: scores + rows ids + 32 staged rows; global route (rows too wide): scores + norms + row ids
-    const size_t head = (size_t)((a.dim + 1) & ~1) * 8;
-    const size_t staged = head + (size_t)cap * 8 + (size_t)((cap + 3) & ~3) * 4 + (size_t)32 * ((size_t)a.ld * dtype_size(a.dtype) + 16) + 64;
-    const int stage_rows = staged <= 200 * 1024 ? 32 : 0;
-    const size_t smem = stage_rows ? staged : head + (size_t)cap * (8 + 8 + 4) + 32;
-    VM_REQUIRE(smem <= 200 * 1024, VM_ERR_UNSUPPORTED, "collect pass: buffer of %d rows exceeds shared memory", cap);
+    // query, scores and row ids of the gathered rows, then the staged-row window
+    constexpr size_t CR_SMEM_LIMIT = 200 * 1024;
+    const size_t fixed = (size_t)((a.dim + 1) & ~1) * 8 + (size_t)cap * 8 + (size_t)((cap + 3) & ~3) * 4 + 64;
+    const StageWindow win = fixed < CR_SMEM_LIMIT ? stage_window(CR_ROWS, a.dtype, a.ld, CR_SMEM_LIMIT - fixed) : StageWindow{0, 0};
+    VM_REQUIRE(win.chunks > 0, VM_ERR_UNSUPPORTED, "collect pass: buffer of %d rows exceeds shared memory", cap);
+    const size_t smem = fixed + (size_t)CR_ROWS * win.pitch;
     return with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
         using T = std::remove_pointer_t<decltype(tag)>;
         constexpr bool NEU = decltype(neu)::value;
         VM_CUDA_CHECK((max_smem_once<collect_rescore_kernel<NEU, T>>(200 * 1024)));
         collect_rescore_kernel<NEU, T><<<a.nq, CR_THREADS, smem, st>>>(buf, cnt, cap, (const T *)a.rows, a.ld, a.dim, a.queries,
-                                                                       a.q_dtype, a.fin, a.flags, a.uncertified_count, a.nq, a.cum, stage_rows);
+                                                                       a.q_dtype, a.fin, a.flags, a.uncertified_count, a.nq, a.cum,
+                                                                       win.pitch, win.chunks);
         VM_CUDA_CHECK(cudaGetLastError());
         return VM_OK;
     });

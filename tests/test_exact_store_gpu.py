@@ -134,8 +134,9 @@ def test_exact_store_rows_the_shadow_cannot_hold(vm):
     st.close()
 
 
-def test_exact_store_wide_rows_take_the_two_kernel_rescoring(vm):
-    """1536-d binary64 rows: 32 candidate rows no longer fit the fused kernel's shared memory."""
+def test_exact_store_wide_rows_take_the_fused_rescoring(vm):
+    """1536-d binary64 rows: 32 whole candidate rows do not fit shared memory, so the rescoring kernel streams them through
+    its window of column chunks."""
     d, n, k = 1536, 12_000, 10
     rng = np.random.default_rng(8)
     X = rng.standard_normal((n, d))
