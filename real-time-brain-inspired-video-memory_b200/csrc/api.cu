@@ -63,7 +63,6 @@ static constexpr int MAXQ = 64;   // queries per scan pass
 static constexpr int MAXK = 64;   // k and candidate-list bound
 static constexpr int XCTAS = 148; // exact-scan grid
 static constexpr int MAX_DEVICES = 64;
-static constexpr int COLLECT_CAP = 4096;         // rows per query the collect pass may gather
 static constexpr int FLAG_INTERNAL_CAPTURE = 1 << 30;  // set by the CUDA-graph path while capturing
 
 // The top-k results of a batch as one contiguous block [idx nq*k i64 | score nq*k f64 | count nq i32], so that one

@@ -7,6 +7,7 @@
 #include <math.h>
 #include <utility>
 #include "../../include/vidmem.h"
+#include "stage_window.h"  // SELECT_KEY_CAP, SCAN_DUMP_TILE, SCAN_DUMP_MAX_KEYS, COLLECT_CAP
 
 namespace vm {
 
@@ -249,9 +250,6 @@ struct ScanArgs {
 };
 static constexpr int SCAN_UNION_CAP = 16384; // shared spill-buffer entries per query (filtered with the final bound before staging)
 static constexpr int SCAN_SLAB = 128;         // keys per (CTA, query) slab
-static constexpr int SELECT_KEY_CAP = 4096;   // band keys the rescoring kernel stages per query after the final filter
-static constexpr int SCAN_DUMP_TILE = 128;     // rows (= keys per query) per dumped tile
-static constexpr int SCAN_DUMP_MAX_KEYS = 9472;  // per query: what the fused select kernel ranks in shared memory (148 x 64)
 int launch_scan_simt(const ScanArgs &a);
 int scan_simt_max_queries();
 // second pass of the tcgen05 scan for uncertified queries (see scan_tc.cu "collect mode")

@@ -10,7 +10,6 @@ namespace vm {
 // =========================================================================================
 // 1. fused candidate selection + exact rescoring + band settlement (ONE launch)
 // =========================================================================================
-static constexpr int SR_THREADS = 512;
 static constexpr int MERGE_SURV = 1024;  // survivors ranked directly
 
 // Exact kp-th largest key of skeys[0..total) by MSB-first radix select (8 passes x 8 bits, shared-memory histogram + one
@@ -79,12 +78,6 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc)
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-// Rows of one query's near-tie band the rescoring kernel settles itself: as many as shared memory leaves room for
-// (12 bytes each), between BAND_CAP_MIN and BAND_CAP_MAX.  Settling 2048 rows costs ~0.3 ms for the batch (64 staged
-// sub-batches per query, the queries in parallel) and no extra pass over the store; bands of up to 4096 rows are left
-// to the collect pass (a second streaming scan + its own rescoring), anything larger to the binary64 scan.
-static constexpr int BAND_CAP_MIN = 1024, BAND_CAP_MAX = 2048;
-
 // Exact top-k among m rows with reference scores s_sc (block-wide): every row is ranked by counting the rows that beat it
 // (score desc, row asc: rows are distinct, so ranks are) and the first k are emitted.  Returns the number of entries
 // emitted (uniform).
@@ -128,7 +121,7 @@ static constexpr uint32_t NO_ROW = 0xFFFFFFFFu;
 // of every row -- through a ring of three slots: slot b starts at group b*win/3 of a staged row of `pitch` = 16*(win+1)
 // bytes.  The chains run over chunk c while chunks c+1 and c+2 load; then chunk c+3 goes into the slot chunk c frees.
 // Three chunks with win = gpr are whole rows, every chunk in its own columns.  Each chain still runs over the columns in
-// index order.  Block-wide; ends with a barrier.
+// index order.  The window (pitch, chunks) comes from stage_window (stage_window.h).  Block-wide; ends with a barrier.
 template <bool NEUMAIER, typename T, int THREADS>
 __device__ __forceinline__ void stage_and_chain(const T *__restrict__ rows, int ld, int dim, int kp, const uint32_t *s_rid,
                                                 unsigned char *srow, int pitch, int chunks, const double *sq, double *s_dot,
@@ -137,8 +130,8 @@ __device__ __forceinline__ void stage_and_chain(const T *__restrict__ rows, int 
     const int tid = threadIdx.x, j = tid;
     const int gpr = ld * (int)sizeof(T) / 16;                 // 16-byte groups per row
     const int win = pitch / 16 - 1;                           // 16-byte groups per staged row
-    auto g_lo = [&](int c) { return c * gpr / chunks; };      // first group of chunk c
-    auto slot = [&](int c) { return (c % 3) * win / 3; };     // first staged group of chunk c's slot
+    auto g_lo = [&](int c) { return stage_chunk_lo(c, gpr, chunks); };  // first group of chunk c
+    auto slot = [&](int c) { return stage_slot_lo(c, win); };           // first staged group of chunk c's slot
     auto issue = [&](int c) {
         const int lo = g_lo(c), w = g_lo(c + 1) - lo, base = slot(c);
         for (int e = tid; e < kp * w; e += THREADS) {
@@ -571,7 +564,6 @@ __global__ void __launch_bounds__(SR_THREADS, 1) select_rescore_kernel(SelectSrc
 // are emitted; the query's flag is cleared.  If the buffer overflowed the flag becomes 2 and the binary64 scan of every
 // row takes over.
 static constexpr int CR_THREADS = 512;
-static constexpr int CR_ROWS = 32;  // rows staged at a time
 template <bool NEUMAIER, typename T>
 __global__ void __launch_bounds__(CR_THREADS, 1) collect_rescore_kernel(const uint64_t *__restrict__ buf, const int *__restrict__ cnt, int cap,
                                                                        const T *__restrict__ rows, int ld, int dim,
@@ -1075,47 +1067,11 @@ static int with_row_type(int dtype, int sum_mode, F &&f)
     return by_sum((__nv_bfloat16 *)nullptr);
 }
 
-// The staged-row window of stage_and_chain for `rows` rows in `room` bytes of shared memory: whole rows in three chunks
-// when they fit (one 16-byte group of padding per row), else the fewest chunks whose three slots fit.  The windowed
-// pitch is an odd number of 16-byte groups, as whole fp32 / binary64 rows are, so that the chains, each walking its own
-// row at the same column, spread over the shared-memory banks.  chunks == 0: not even one group per slot fits.
-struct StageWindow { int pitch, chunks; };
-static StageWindow stage_window(int rows, int dtype, int ld, size_t room)
-{
-    const int gpr = ld * (int)dtype_size(dtype) / 16;        // 16-byte groups per row
-    if ((size_t)rows * (gpr + 1) * 16 <= room) return {(gpr + 1) * 16, 3};
-    for (int chunks = 4; chunks <= gpr; ++chunks) {
-        const int s = (gpr + chunks - 1) / chunks;           // groups of the widest chunk
-        const int win = 3 * s + (s & 1);                     // three slots of >= s groups, win + 1 odd
-        if ((size_t)rows * (win + 1) * 16 <= room) return {(win + 1) * 16, chunks};
-    }
-    return {0, 0};
-}
-
-// Shared memory of select_rescore_kernel: keys, list maxima, query and the staged-row window, sized to leave room for at
-// least BAND_CAP_MIN band rows; then as many band rows (12 bytes each) as fit, up to BAND_CAP_MAX.  band_cap == 0: the
-// shape does not fit.
-static constexpr size_t SR_SMEM_LIMIT = 180 * 1024;
-struct SelectLayout { StageWindow win; int band_cap; size_t smem; };
-static SelectLayout select_layout(int key_cap, int lists, int kp, int dtype, int dim, int ld)
-{
-    const size_t fixed = (size_t)key_cap * 8 + (size_t)((lists + 3) & ~3) * 4 + (size_t)((dim + 1) & ~1) * 8 + 16 + 32;
-    const size_t need = fixed + (size_t)BAND_CAP_MIN * 12;
-    SelectLayout L{{0, 0}, 0, 0};
-    if (need > SR_SMEM_LIMIT) return L;
-    L.win = stage_window(kp, dtype, ld, SR_SMEM_LIMIT - need);
-    if (L.win.chunks == 0) return L;
-    const size_t base = fixed + (size_t)kp * L.win.pitch;
-    const size_t cap = ((SR_SMEM_LIMIT - base) / 12) & ~(size_t)63;
-    L.band_cap = (int)(cap < (size_t)BAND_CAP_MAX ? cap : (size_t)BAND_CAP_MAX);
-    L.smem = base + (size_t)L.band_cap * 12;
-    return L;
-}
 // lists == 0: slab mode (tcgen05 scan); else list mode with lists x list_len keys per query
 bool select_rescore_fits(int lists, int list_len, int kp, int dtype, int dim, int ld)
 {
     const int key_cap = lists > 0 ? lists * list_len : SELECT_KEY_CAP;
-    return select_layout(key_cap, lists, kp, dtype, dim, ld).band_cap >= BAND_CAP_MIN && kp <= 64 && 2 * kp + 1 <= SR_THREADS;
+    return select_layout_fits(key_cap, lists, kp, (int)dtype_size(dtype), dim, ld);
 }
 
 static SelectSrc make_src(const SelectArgs &sa)
@@ -1132,14 +1088,14 @@ int k_select_rescore(const SelectArgs &sa, const RescoreArgs &a, cudaStream_t st
     VM_REQUIRE(src.slab == nullptr || src.ctas <= 256, VM_ERR_UNSUPPORTED, "select: %d scan CTAs exceed 256", src.ctas);
     VM_REQUIRE(select_rescore_fits(src.lists, src.list_len, a.kp, a.dtype, a.dim, a.ld), VM_ERR_UNSUPPORTED,
                "select: %d keys and %d candidate rows of %d columns exceed shared memory", src.key_cap, a.kp, a.dim);
-    const SelectLayout L = select_layout(src.key_cap, src.lists, a.kp, a.dtype, a.dim, a.ld);
+    const SelectLayout L = select_layout(src.key_cap, src.lists, a.kp, (int)dtype_size(a.dtype), a.dim, a.ld);
     src.band_cap = L.band_cap;
     src.pitch = L.win.pitch;
     src.chunks = L.win.chunks;
     return with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
         using T = std::remove_pointer_t<decltype(tag)>;
         constexpr bool NEU = decltype(neu)::value;
-        VM_CUDA_CHECK((max_smem_once<select_rescore_kernel<NEU, T>>(180 * 1024)));
+        VM_CUDA_CHECK((max_smem_once<select_rescore_kernel<NEU, T>>((int)SR_SMEM_LIMIT)));
         VM_CUDA_CHECK(launch_pdl(select_rescore_kernel<NEU, T>, dim3(a.nq), dim3(SR_THREADS), L.smem, st, pdl, src, a.nq, a.kp,
                                  (const T *)a.rows, a.ld, a.dim, a.n_rows, a.queries, a.q_dtype, a.eps, a.fin, a.flags,
                                  a.uncertified_count, a.extreme, a.collect_thr, a.cum, a.inv_norms));
@@ -1150,16 +1106,14 @@ int k_select_rescore(const SelectArgs &sa, const RescoreArgs &a, cudaStream_t st
 
 int k_collect_rescore(const uint64_t *buf, const int *cnt, int cap, const RescoreArgs &a, cudaStream_t st)
 {
-    // query, scores and row ids of the gathered rows, then the staged-row window
-    constexpr size_t CR_SMEM_LIMIT = 200 * 1024;
-    const size_t fixed = (size_t)((a.dim + 1) & ~1) * 8 + (size_t)cap * 8 + (size_t)((cap + 3) & ~3) * 4 + 64;
-    const StageWindow win = fixed < CR_SMEM_LIMIT ? stage_window(CR_ROWS, a.dtype, a.ld, CR_SMEM_LIMIT - fixed) : StageWindow{0, 0};
+    const CollectLayout L = collect_layout(cap, (int)dtype_size(a.dtype), a.dim, a.ld);
+    const StageWindow win = L.win;
     VM_REQUIRE(win.chunks > 0, VM_ERR_UNSUPPORTED, "collect pass: buffer of %d rows exceeds shared memory", cap);
-    const size_t smem = fixed + (size_t)CR_ROWS * win.pitch;
+    const size_t smem = L.smem;
     return with_row_type(a.dtype, a.sum_mode, [&](auto neu, auto *tag) -> int {
         using T = std::remove_pointer_t<decltype(tag)>;
         constexpr bool NEU = decltype(neu)::value;
-        VM_CUDA_CHECK((max_smem_once<collect_rescore_kernel<NEU, T>>(200 * 1024)));
+        VM_CUDA_CHECK((max_smem_once<collect_rescore_kernel<NEU, T>>((int)CR_SMEM_LIMIT)));
         collect_rescore_kernel<NEU, T><<<a.nq, CR_THREADS, smem, st>>>(buf, cnt, cap, (const T *)a.rows, a.ld, a.dim, a.queries,
                                                                        a.q_dtype, a.fin, a.flags, a.uncertified_count, a.nq, a.cum,
                                                                        win.pitch, win.chunks);
