@@ -117,8 +117,8 @@ int vm_store_attach(vm_store **out, int device, int dim, int dtype, int64_t capa
 /* BINARY64 store: the rows are kept exactly as given (the reference scores Python float lists, i.e. binary64:
  * pre_llm_injector.py:382-388), [capacity][ld] doubles, next to a rounded SHADOW copy in `shadow_dtype` (VM_F32 or
  * VM_BF16) that only the streaming scan reads.  Candidate selection runs on the shadow with an error bound widened
- * by the shadow's rounding (2^-24 / 2^-9 in cosine units); every exact step -- rescoring, near-tie band, collect pass,
- * binary64 scan -- reads the binary64 rows.  Returned scores and order are therefore those of the reference formula on
+ * by the shadow's rounding (2^-24 / 2^-8 in cosine units, with margin); every exact step -- rescoring, near-tie band,
+ * collect pass, binary64 scan -- reads the binary64 rows.  Returned scores and order are therefore those of the reference formula on
  * the ORIGINAL values, whatever their representability in fp32 / bf16.  HBM per row: ld * (8 + sizeof(shadow)) + 4
  * bytes; scan traffic is that of the shadow alone.  vm_store_attach_exact: rows_exact_dev holds capacity * vm_ld(dim)
  * doubles (16-byte aligned).  Rows whose elements overflow the shadow type, or that vanish in it, stay scorable: they

@@ -1,6 +1,7 @@
 // api.cu -- the C ABI of libvidmem.so (include/vidmem.h): handles, workspaces, orchestration of
 // scan -> merge -> exact rescoring -> (rare) exact re-scan, NCCL gather + merge for shards.
 #include "common.cuh"
+#include "scan_eps.h"
 
 #include <dlfcn.h>
 #include <stdarg.h>
@@ -291,30 +292,6 @@ static int ws_prepare(vm_store *s)
     VM_CUDA_CHECK(cudaMallocHost((void **)&w.h_q, (size_t)MAXQ * s->dim * 8));
     w.ready = true;
     return VM_OK;
-}
-
-static double scan_eps_stored(int kernel, int store_dtype, int dim, int split);
-// shadow: the store keeps binary64 originals and the scan reads their rounded copy.  Rounding a row moves its
-// direction by an angle of at most asin(u) (u = unit roundoff of the shadow type, relative per element, hence relative
-// in norm), and a cosine moves by at most the angle: + 2^-24 (fp32 shadow) or + 2^-9 (bf16 shadow), taken with margin.
-static double scan_eps(int kernel, int store_dtype, int dim, int split, bool shadow = false)
-{
-    const double base = scan_eps_stored(kernel, store_dtype, dim, split);
-    if (!shadow) return base;
-    return base + (store_dtype == VM_F32 ? 1.1920928955078125e-07 : 1.953125e-3 * 1.01);
-}
-static double scan_eps_stored(int kernel, int store_dtype, int dim, int split)
-{
-    // Bound on |approximate cosine - exact cosine| (DESIGN.md "certification"), in cosine units (Cauchy-Schwarz).
-    const double u = 1.1920928955078125e-07;                         // 2^-23
-    const double fp32_acc = (double)(dim + 16) * u;                  // fp32 accumulation + normalisation of query and row
-    if (kernel == 1) return fp32_acc;                                // CUDA-core fp32 scan
-    if (store_dtype == VM_F32)                                       // tf32: rows truncated (2^-10), query pre-rounded to nearest (2^-11)
-        return 9.765625e-4 + 4.8828125e-4 + 1e-6 + fp32_acc;
-    if (!split) return 3.90625e-3 + fp32_acc;                        // bf16 store (exact operand), query rounded to bf16: 2^-8
-    // bf16 store, query = hi + lo: residual 2^-16; the lo products are 2^-8 of the hi ones, their MMAs add one
-    // accumulator rounding each (dim/16 of them) -- counted generously as dim/8 + 16 extra terms
-    return 1.52587890625e-5 * 1.01 + (double)(dim + dim / 8 + 32) * u;
 }
 
 // ---- library --------------------------------------------------------------------------------

@@ -17,6 +17,7 @@
 // pairs_finalize_kernel, so the emitted pair SET is exact for the stored values.
 #include "tc_common.cuh"
 #include "raster.h"
+#include "scan_eps.h"
 #include <stdlib.h>
 #include <mutex>
 
@@ -519,8 +520,7 @@ int k_pairs_above(int device, const void *x, int dtype, int64_t n, int dim, int 
     if (rc != VM_OK) return rc;
 
     const int es = dtype == VM_F32 ? 4 : 2;
-    const float fp32_acc = (float)(dim + 32) * 1.1920928955078125e-07f;
-    const float eps = dtype == VM_F32 ? 3.90625e-3f + fp32_acc : fp32_acc;  // tf32: both operands truncated twice over i and j
+    const float eps = pairs_eps(dtype, dim);
     PairsParams p{};
     p.n = n;
     p.nbi = (int)((n + P_BM - 1) / P_BM);
